@@ -133,6 +133,13 @@ int svb_launch_count_end(long long* ours, long long* other, char* names, size_t 
 
 /* ---- GE2E loss (speech_embedder_net.py:35-49, utils.py:27-132) ---------------------------------------------------- */
 
+/* GE2E loss methods (Wan et al., arXiv 1710.10467):
+ *   SVB_GE2E_SOFTMAX  eq. 6, the reference's calc_loss (utils.py:126-132): per = -S_jj + log(sum_k exp S_jk + 1e-6);
+ *   SVB_GE2E_CONTRAST eq. 7: per = 1 - sigmoid(S_jj) + sigmoid(S_jk*), k* = argmax_{k != j} S_jk (lowest index among
+ *                     ties).  Needs at least two centroid columns.  The loss is the SUM over rows for both. */
+#define SVB_GE2E_SOFTMAX 0
+#define SVB_GE2E_CONTRAST 1
+
 int svb_ge2e_workspace_bytes(int N, int M, int D, int Nc, size_t* bytes);
 /* Debug (env SVB_GE2E_TRACE=1): byte offset inside the workspace of the per-speaker kernel's clock64 phase stamps,
  * [CTA][16] int64 (scripts/trace_ge2e.py). */
@@ -151,6 +158,13 @@ int svb_ge2e_trace_offset(int N, int M, int D, int Nc, size_t* offset);
 int svb_ge2e(const float* E, const float* Cext, int N, int M, int D, int Nc, const float* w, const float* b,
              const float* dcos, const float* gscale, float* cos_out, float* per_out, float* loss_out, float* dE,
              float* dCext, float* dw, float* db, void* workspace, size_t workspace_bytes, int fused, void* stream);
+/* svb_ge2e with a loss method (SVB_GE2E_*); svb_ge2e is svb_ge2e_ex(..., SVB_GE2E_SOFTMAX, stream).  The contrast
+ * method is a loss: it needs w and b, and has no cosine-only or dcos mode.  Its backward gathers one centroid per row
+ * (no dense A_off products); the workspace size is the same. */
+int svb_ge2e_ex(const float* E, const float* Cext, int N, int M, int D, int Nc, const float* w, const float* b,
+                const float* dcos, const float* gscale, float* cos_out, float* per_out, float* loss_out, float* dE,
+                float* dCext, float* dw, float* db, void* workspace, size_t workspace_bytes, int fused, int loss,
+                void* stream);
 
 /* Row shard of a global GE2E batch (new: multi-GPU, one process per GPU; the reference is single-device).  E: the M
  * utterances of speakers [col0, col0 + N_local) of a batch of Nc speakers; C (Nc, D): all centroids (utils.py:27-29 of
@@ -162,6 +176,10 @@ int svb_ge2e(const float* E, const float* Cext, int N, int M, int D, int Nc, con
 int svb_ge2e_rows(const float* E, const float* C, int N_local, int M, int D, int Nc, int col0, const float* w,
                   const float* b, const float* gscale, float* per_out, float* loss_out, float* dE, float* dC, float* dw,
                   float* db, void* workspace, size_t workspace_bytes, void* stream);
+/* svb_ge2e_rows with a loss method (SVB_GE2E_*). */
+int svb_ge2e_rows_ex(const float* E, const float* C, int N_local, int M, int D, int Nc, int col0, const float* w,
+                     const float* b, const float* gscale, float* per_out, float* loss_out, float* dE, float* dC,
+                     float* dw, float* db, void* workspace, size_t workspace_bytes, int loss, void* stream);
 
 /* utils.get_centroids (utils.py:27-29) and its backward. */
 int svb_centroids(const float* E, float* C, int N, int M, int D, void* stream);
@@ -175,6 +193,9 @@ int svb_utterance_centroids(const float* E, float* U, int N, int M, int D, void*
 /* utils.calc_loss (utils.py:126-132) on a caller-supplied similarity matrix S (N,M,Nc); dS optional. */
 int svb_calc_loss(const float* S, int N, int M, int Nc, float* per_out, float* loss_out, float* dS,
                   const float* gscale, void* stream);
+/* svb_calc_loss with a loss method (SVB_GE2E_*): dS = gscale * dL/dS of that method. */
+int svb_calc_loss_ex(const float* S, int N, int M, int Nc, float* per_out, float* loss_out, float* dS,
+                     const float* gscale, int loss, void* stream);
 
 /* x[i] *= *g for three buffers in one launch (autograd's upstream scalar). */
 int svb_scale3(float* a, size_t na, float* b, size_t nb, float* c, size_t nc, const float* g, void* stream);

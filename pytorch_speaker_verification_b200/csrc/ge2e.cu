@@ -35,6 +35,8 @@ constexpr float kCosBias = 1e-6f;   // utils.py:114
 constexpr float kLogBias = 1e-6f;   // utils.py:129
 constexpr int kThreads = 256;
 constexpr int kWarps = kThreads / 32;
+constexpr int kSoftmax = SVB_GE2E_SOFTMAX;    // loss method of the row phase (template argument of the loss kernels)
+constexpr int kContrast = SVB_GE2E_CONTRAST;
 
 struct Ge2eArgs {
   const float* E;        // [N, M, D]
@@ -92,6 +94,31 @@ __device__ __forceinline__ float warp_max(float v) {
   for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
 }
+// Arg-max over (value, index) pairs across the warp: the larger value wins, equal values keep the lower index (the
+// element torch.max returns); k < 0 marks a lane without a candidate.  Every lane ends with the same pair.
+__device__ __forceinline__ void warp_argmax(float& v, int& k) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, v, o);
+    const int ok = __shfl_xor_sync(0xffffffffu, k, o);
+    if (ok >= 0 && (k < 0 || ov > v || (ov == v && ok < k))) { v = ov; k = ok; }
+  }
+}
+__device__ __forceinline__ float sigmoid(float x) { return 1.0f / (1.0f + expf(-x)); }
+// GE2E contrast loss of one row (Wan et al. eq. 7): per = 1 - sig(S_jj) + sig(S_jk*), k* = argmax_{k != j} S_jk.
+// G_jj = -sig(S_jj) sig(-S_jj), G_jk* = sig(S_jk*) sig(-S_jk*), every other G is 0 (1 - sig(x) is evaluated as sig(-x)).
+struct ContrastRow {
+  float per, gd, gk;
+};
+__device__ __forceinline__ ContrastRow contrast_row(float sd, float sk) {
+  const float pd = sigmoid(sd), nd = sigmoid(-sd), pk = sigmoid(sk), nk = sigmoid(-sk);
+  return ContrastRow{nd + pk, -pd * nd, pk * nk};
+}
+// The contrast loss keeps one non-zero of A_off per row: its column k* and value w G_jk* live in the (otherwise unused)
+// dense A_off slot of the workspace: [NM] ints, then [NM] floats.
+__device__ __forceinline__ int* contrast_kstar(const Ge2eArgs& a) { return reinterpret_cast<int*>(a.Aoff); }
+__device__ __forceinline__ float* contrast_gstar(const Ge2eArgs& a) { return a.Aoff + (size_t)a.N * a.M; }
+
 // Block-wide sum, result broadcast to every thread.  red must hold kWarps floats.
 __device__ float block_sum(float v, float* red) {
   v = warp_sum(v);
@@ -261,7 +288,10 @@ __device__ void phase_b1(const Ge2eArgs& a, float* smem) {
 }
 
 // ---------------------------------------------------------------------------------------------- phase B2: row softmax
-// one warp per embedding row: diagonal overwrite, S = w cos + b, stable log-sum-exp, G, A = w G (diag split off)
+// one warp per embedding row: diagonal overwrite, S = w cos + b, stable log-sum-exp, G, A = w G (diag split off).
+// LOSS = kContrast: arg-max k* over the off-diagonal S instead, G has two non-zeros; no dense A_off is written, only
+// (k*, w G_jk*) per row for the gather backward of phase D.
+template <int LOSS>
 __device__ void phase_b2(const Ge2eArgs& a) {
   const int M = a.M, Nc = a.Nc, NM = a.N * a.M;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -274,7 +304,27 @@ __device__ void phase_b2(const Ge2eArgs& a) {
     __syncwarp();
     if (a.cos_out)
       for (int k = lane; k < Nc; k += 32) a.cos_out[(size_t)row * Nc + k] = t[k] + kCosBias;
-    if (a.w) {
+    if (LOSS == kContrast) {                            // (loss mode only: the host requires w, b)
+      float sk = -INFINITY;
+      int ks = -1;
+      for (int k = lane; k < Nc; k += 32) {
+        if (k == j) continue;
+        const float s = w * (t[k] + kCosBias) + b;
+        if (ks < 0 || s > sk) { sk = s; ks = k; }
+      }
+      warp_argmax(sk, ks);
+      if (lane == 0) {
+        const float cd1 = cd + kCosBias, ck1 = t[ks] + kCosBias;
+        const ContrastRow c = contrast_row(w * cd1 + b, sk);
+        a.rowstat[row] = c.per;
+        a.rowstat[NM + row] = c.gd * cd1 + c.gk * ck1;
+        a.rowstat[2 * NM + row] = c.gd + c.gk;
+        if (a.per_out) a.per_out[row] = c.per;
+        a.adiag[row] = w * c.gd;
+        contrast_kstar(a)[row] = ks;
+        contrast_gstar(a)[row] = w * c.gk;
+      }
+    } else if (a.w) {
       float mx = -INFINITY;
       for (int k = lane; k < Nc; k += 32) mx = fmaxf(mx, w * (t[k] + kCosBias) + b);
       mx = warp_max(mx);
@@ -357,6 +407,43 @@ __device__ float sum_slices(const float* p, size_t stride, int n) {
   for (; i < n; ++i) v += p[(size_t)i * stride];
   return v;
 }
+// Contrast loss, gather form of P_k = sum_rows A_off[row, k] e^_row: P[d] += sum of w G_jk* e^_row[d] over the rows whose
+// k* is k, added in row order (one pass over k*; the matching rows of each 256-row chunk are compacted in order into
+// lst / lg, then every thread adds them to its own dimensions).  Called by the whole block.
+__device__ void contrast_gather_p(const Ge2eArgs& a, int k, float* P, int* lst, float* lg, int* wcnt) {
+  const int NM = a.N * a.M, D = a.D;
+  const int* ks = contrast_kstar(a);
+  const float* gst = contrast_gstar(a);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int r0 = 0; r0 < NM; r0 += kThreads) {
+    const int r = r0 + threadIdx.x;
+    const bool hit = r < NM && ks[r] == k;
+    const unsigned bal = __ballot_sync(0xffffffffu, hit);
+    __syncthreads();                                   // the previous chunk's list is consumed
+    if (lane == 0) wcnt[warp] = __popc(bal);
+    __syncthreads();
+    int base = 0, tot = 0;
+#pragma unroll
+    for (int i = 0; i < kWarps; ++i) {
+      base += i < warp ? wcnt[i] : 0;
+      tot += wcnt[i];
+    }
+    if (tot == 0) continue;
+    if (hit) {
+      const int p = base + __popc(bal & ((1u << lane) - 1u));
+      lst[p] = r;
+      lg[p] = gst[r];
+    }
+    __syncthreads();
+    for (int d = threadIdx.x; d < D; d += kThreads) {
+      float v = P[d];
+      for (int i = 0; i < tot; ++i) v += lg[i] * a.Ehat[(size_t)lst[i] * D + d];
+      P[d] = v;
+    }
+  }
+}
+// LOSS = kContrast: R_row = w G_jk* c^_k* and P_j from contrast_gather_p (no phase C products)
+template <int LOSS>
 __device__ void phase_d(const Ge2eArgs& a, float* smem) {
   const int M = a.M, D = a.D, NM = a.N * a.M;
   float* red = smem;                 // [kWarps]
@@ -366,6 +453,8 @@ __device__ void phase_d(const Ge2eArgs& a, float* smem) {
   float* rE = vec + 3 * D;           // [M, D] e
   float* rH = rE + (size_t)M * D;    // [M, D] e^
   float* rR = rH + (size_t)M * D;    // [M, D] R
+  float* lg = rR + (size_t)M * D;    // contrast: [kThreads] w G_jk* of the compacted rows
+  int* lst = reinterpret_cast<int*>(lg + kThreads);   // contrast: [kThreads] their row indices, then [kWarps] counts
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const float gs = a.gscale ? *a.gscale : 1.0f;
   if (a.need_grad) {
@@ -377,10 +466,16 @@ __device__ void phase_d(const Ge2eArgs& a, float* smem) {
       for (int i = threadIdx.x; i < M * D; i += kThreads) {
         rE[i] = a.E[row0 * D + i];
         rH[i] = a.Ehat[row0 * D + i];
-        rR[i] = a.R[row0 * D + i];
+        if (LOSS == kContrast) {
+          const size_t row = row0 + i / D;
+          rR[i] = contrast_gstar(a)[row] * a.Chat[(size_t)contrast_kstar(a)[row] * D + i % D];
+        } else {
+          rR[i] = a.R[row0 * D + i];
+        }
       }
       for (int d = threadIdx.x; d < D; d += kThreads) {
-        vec[d] = a.Cext ? 0.f : sum_slices(a.dC + (size_t)j * D + d, pstride, a.psplit);
+        if (LOSS == kContrast) vec[d] = 0.f;
+        else vec[d] = a.Cext ? 0.f : sum_slices(a.dC + (size_t)j * D + d, pstride, a.psplit);
         vec[D + d] = a.Cext ? 0.f : a.Chat[(size_t)j * D + d];
         vec[2 * D + d] = a.Ssum[(size_t)j * D + d];
       }
@@ -388,6 +483,7 @@ __device__ void phase_d(const Ge2eArgs& a, float* smem) {
         sc[m] = a.inv_ne[row0 + m]; sc[M + m] = a.inv_nu[row0 + m];
         sc[2 * M + m] = a.cosd[row0 + m]; sc[3 * M + m] = a.adiag[row0 + m];
       }
+      if (LOSS == kContrast && !a.Cext) contrast_gather_p(a, j, vec, lst, lg, lst + kThreads);
       __syncthreads();
       float q = 0.f;
       for (int d = threadIdx.x; d < D; d += kThreads) q += vec[d] * vec[D + d];
@@ -420,7 +516,19 @@ __device__ void phase_d(const Ge2eArgs& a, float* smem) {
       }
       __syncthreads();
     }
-    if (a.Cext && a.dCext) {    // gradient w.r.t. foreign centroids: (P_k - (P_k.c^_k) c^_k)/|c_k|, one warp per k
+    if (LOSS == kContrast && a.Cext && a.dCext) {   // the same for the contrast loss, one block per k
+      for (int k = blockIdx.x; k < a.Nc; k += gridDim.x) {
+        __syncthreads();                                   // vec is free
+        for (int d = threadIdx.x; d < D; d += kThreads) vec[d] = 0.f;
+        contrast_gather_p(a, k, vec, lst, lg, lst + kThreads);
+        __syncthreads();
+        float q = 0.f;
+        for (int d = threadIdx.x; d < D; d += kThreads) q += vec[d] * a.Chat[(size_t)k * D + d];
+        q = block_sum(q, red);
+        for (int d = threadIdx.x; d < D; d += kThreads)
+          a.dCext[(size_t)k * D + d] = gs * (vec[d] - q * a.Chat[(size_t)k * D + d]) * a.inv_nc[k];
+      }
+    } else if (a.Cext && a.dCext) {    // gradient w.r.t. foreign centroids: (P_k - (P_k.c^_k) c^_k)/|c_k|, one warp per k
       for (int k = blockIdx.x * kWarps + warp; k < a.Nc; k += gridDim.x * kWarps) {
         float q = 0.f;
         const size_t pstr = (size_t)a.Nc * D;
@@ -452,13 +560,25 @@ __global__ void __launch_bounds__(kThreads) ge2e_fused_kernel(const Ge2eArgs a) 
   grid.sync();
   phase_b1(a, smem);
   grid.sync();
-  phase_b2(a);
+  phase_b2<kSoftmax>(a);
   if (a.need_grad) {
     grid.sync();
     phase_c(a, smem);
   }
   grid.sync();
-  phase_d(a, smem);
+  phase_d<kSoftmax>(a, smem);
+}
+// Contrast loss: phase C (the two dense products R = A_off C^, P = A_off^T E^) is replaced by the gathers of phase D.
+__global__ void __launch_bounds__(kThreads) ge2e_fused_contrast_kernel(const Ge2eArgs a) {
+  extern __shared__ float smem[];
+  cg::grid_group grid = cg::this_grid();
+  phase_a(a, smem);
+  grid.sync();
+  phase_b1(a, smem);
+  grid.sync();
+  phase_b2<kContrast>(a);
+  grid.sync();
+  phase_d<kContrast>(a, smem);
 }
 // One kernel per phase (multi-launch forms): each phase gets its own register allocation and occupancy (as one kernel
 // with a run-time phase switch every phase ran at the 164 registers of the widest one: one CTA per SM).
@@ -467,9 +587,16 @@ __global__ void __launch_bounds__(kThreads) ge2e_phase_kernel(const Ge2eArgs a) 
   extern __shared__ float smem[];
   if (PHASE == 0) phase_a(a, smem);
   else if (PHASE == 1) phase_b1(a, smem);
-  else if (PHASE == 2) phase_b2(a);
+  else if (PHASE == 2) phase_b2<kSoftmax>(a);
   else if (PHASE == 3) phase_c(a, smem);
-  else phase_d(a, smem);
+  else phase_d<kSoftmax>(a, smem);
+}
+// Contrast loss: its row phase (PHASE 2) and phase D (PHASE 4); phases A and B1 are the kernels above.
+template <int PHASE>
+__global__ void __launch_bounds__(kThreads) ge2e_phase_contrast_kernel(const Ge2eArgs a) {
+  extern __shared__ float smem[];
+  if (PHASE == 2) phase_b2<kContrast>(a);
+  else phase_d<kContrast>(a, smem);
 }
 
 // ---------------------------------------------------------------------------------------------- small-batch kernel
@@ -554,8 +681,10 @@ __device__ __forceinline__ void spk_grid_barrier(unsigned* bar, unsigned nblocks
   __syncthreads();
 }
 
-template <int MP, int CL>
-__global__ void __launch_bounds__(kST, 1) ge2e_speaker_kernel(const Ge2eArgs a) {
+// LOSS = kContrast replaces the softmax block of phase 2 by the contrast row block (one non-zero of A_off per row);
+// everything else, the on-chip R and the P slab included, is shared.
+template <int MP, int CL, int LOSS>
+__device__ __forceinline__ void ge2e_speaker_body(const Ge2eArgs& a) {
   constexpr int MS = (MP + 3) & ~3;       // row stride of the [k][m] arrays (float4 loads)
   extern __shared__ float4 smem4[];
   float* smem = reinterpret_cast<float*>(smem4);
@@ -703,7 +832,33 @@ __global__ void __launch_bounds__(kST, 1) ge2e_speaker_kernel(const Ge2eArgs a) 
     __syncthreads();
   }
   if (a.trace && tid == 0) a.trace[blockIdx.x * 16 + 4] = clock64();
-  {   // softmax: one warp per row (both CTAs of a cluster, identical inputs -> identical A)
+  if constexpr (LOSS == kContrast) {   // contrast: one warp per row (both CTAs of a cluster see identical cosr -> same k*)
+    const float w = *a.w, b = *a.b;
+    for (int m = warp; m < M; m += kSW) {
+      const float* t = cosr + m * L.Npad;
+      float sk = -INFINITY;
+      int ks = -1;
+      for (int k = lane; k < N; k += 32) {
+        if (k == j) continue;
+        const float s = w * (t[k] + kCosBias) + b;
+        if (ks < 0 || s > sk) { sk = s; ks = k; }
+      }
+      warp_argmax(sk, ks);
+      if (lane == 0) {
+        const float cd1 = cosd[m] + kCosBias, ck1 = t[ks] + kCosBias;
+        const ContrastRow c = contrast_row(w * cd1 + b, sk);
+        if (h == 0) {
+          const size_t row = row0 + m;
+          a.rowstat[row] = c.per;
+          a.rowstat[NM + row] = c.gd * cd1 + c.gk * ck1;
+          a.rowstat[2 * NM + row] = c.gd + c.gk;
+          if (a.per_out) a.per_out[row] = c.per;
+        }
+        adiag[m] = w * c.gd;
+        At[ks * MS + m] = w * c.gk;                   // At is zero elsewhere (phase 1)
+      }
+    }
+  } else {   // softmax: one warp per row (both CTAs of a cluster, identical inputs -> identical A)
     const float w = *a.w, b = *a.b;
     for (int m = warp; m < M; m += kSW) {
       const float* t = cosr + m * L.Npad;
@@ -865,6 +1020,14 @@ __global__ void __launch_bounds__(kST, 1) ge2e_speaker_kernel(const Ge2eArgs a) 
     }
   }
 }
+template <int MP, int CL>
+__global__ void __launch_bounds__(kST, 1) ge2e_speaker_kernel(const Ge2eArgs a) {
+  ge2e_speaker_body<MP, CL, kSoftmax>(a);
+}
+template <int MP, int CL>
+__global__ void __launch_bounds__(kST, 1) ge2e_speaker_contrast_kernel(const Ge2eArgs a) {
+  ge2e_speaker_body<MP, CL, kContrast>(a);
+}
 
 static size_t align_up(size_t x) { return (x + 255) & ~size_t(255); }
 
@@ -884,7 +1047,23 @@ static void* spk_kernel_cl(int MP) {
     default: return (void*)ge2e_speaker_kernel<16, CL>;
   }
 }
-static void* spk_kernel(int MP, int CL) { return CL > 1 ? spk_kernel_cl<2>(MP) : spk_kernel_cl<1>(MP); }
+template <int CL>
+static void* spk_contrast_kernel_cl(int MP) {
+  switch (MP) {
+    case 2: return (void*)ge2e_speaker_contrast_kernel<2, CL>;
+    case 4: return (void*)ge2e_speaker_contrast_kernel<4, CL>;
+    case 6: return (void*)ge2e_speaker_contrast_kernel<6, CL>;
+    case 8: return (void*)ge2e_speaker_contrast_kernel<8, CL>;
+    case 10: return (void*)ge2e_speaker_contrast_kernel<10, CL>;
+    case 12: return (void*)ge2e_speaker_contrast_kernel<12, CL>;
+    case 14: return (void*)ge2e_speaker_contrast_kernel<14, CL>;
+    default: return (void*)ge2e_speaker_contrast_kernel<16, CL>;
+  }
+}
+static void* spk_kernel(int MP, int CL, int loss) {
+  if (loss == kContrast) return CL > 1 ? spk_contrast_kernel_cl<2>(MP) : spk_contrast_kernel_cl<1>(MP);
+  return CL > 1 ? spk_kernel_cl<2>(MP) : spk_kernel_cl<1>(MP);
+}
 
 static size_t carve(Ge2eArgs& a, char* base) {
   const size_t NM = (size_t)a.N * a.M, D = a.D, Nc = a.Nc;
@@ -906,10 +1085,11 @@ static size_t carve(Ge2eArgs& a, char* base) {
   return off;
 }
 
-static size_t smem_bytes(const Ge2eArgs& a) {
+static size_t smem_bytes(const Ge2eArgs& a, int loss = kSoftmax) {
   size_t pa = (size_t)a.D + kWarps + (size_t)a.M * a.D;
   size_t pg = (size_t)kTK * (kTM + 4) + (size_t)kTK * (kTN + 4);
   size_t pd = (size_t)kWarps + 5 * (size_t)a.M + 3 * (size_t)a.D + 3 * (size_t)a.M * a.D;
+  if (loss == kContrast) pd += 2 * (size_t)kThreads + kWarps;        // contrast_gather_p's row list and counts
   size_t m = pa > pg ? pa : pg;
   m = m > pd ? m : pd;
   return m * sizeof(float);
@@ -944,8 +1124,11 @@ extern "C" int svb_set_ge2e_tensor_cores(int on) { g_ge2e_tc = on != 0; return S
 static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int Nc, int col0, const float* w,
                      const float* b, const float* dcos, const float* gscale, float* cos_out, float* per_out,
                      float* loss_out, float* dE, float* dCext, float* dw, float* db, void* workspace,
-                     size_t workspace_bytes, int fused, void* stream) {
+                     size_t workspace_bytes, int fused, int loss, void* stream) {
   if (!E || N < 1 || M < 2 || D < 1 || !workspace) { set_error("svb_ge2e: bad argument (M must be >= 2)", cudaSuccess); return SVB_ERR_ARG; }
+  if (loss != kSoftmax && loss != kContrast) { set_error("svb_ge2e: unknown loss method", cudaSuccess); return SVB_ERR_ARG; }
+  if (loss == kContrast && (!w || dcos)) { set_error("svb_ge2e: the contrast loss method needs w and b (no cosine-only or dcos mode)", cudaSuccess); return SVB_ERR_ARG; }
+  if (loss == kContrast && Nc < 2) { set_error("svb_ge2e: the contrast loss needs at least two centroid columns", cudaSuccess); return SVB_ERR_ARG; }
   if (col0 < 0 || (col0 > 0 && (!Cext || col0 + N > Nc))) { set_error("svb_ge2e: row shard outside the centroid matrix", cudaSuccess); return SVB_ERR_ARG; }
   if (!Cext && Nc != N) { set_error("svb_ge2e: Nc must equal N without foreign centroids", cudaSuccess); return SVB_ERR_ARG; }
   if ((w == nullptr) != (b == nullptr)) return SVB_ERR_ARG;
@@ -959,7 +1142,8 @@ static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int
   static const bool trace_on = getenv("SVB_GE2E_TRACE") != nullptr;
   if (!trace_on) a.trace = nullptr;
   const size_t smem = smem_bytes(a);
-  if (smem > 200 * 1024) { set_error("svb_ge2e: M*D too large for one CTA's shared memory", cudaSuccess); return SVB_ERR_UNSUPPORTED; }
+  const size_t smem_ct = smem_bytes(a, loss);           // (== smem for the softmax loss)
+  if (smem_ct > 200 * 1024) { set_error("svb_ge2e: M*D too large for one CTA's shared memory", cudaSuccess); return SVB_ERR_UNSUPPORTED; }
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   static int max_smem_tab[kMaxDevices] = {};          // cudaFuncSetAttribute is per device
   const int dev_i = current_device_index();
@@ -975,6 +1159,15 @@ static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int
     if (e != cudaSuccess) { set_error("svb_ge2e: cudaFuncSetAttribute", e); return SVB_ERR_CUDA; }
     max_smem_set = (int)smem;
   }
+  const bool contrast = loss == kContrast;
+  static int max_smem_ct_tab[kMaxDevices] = {};       // the contrast kernels' own attribute
+  if (contrast && (int)smem_ct > max_smem_ct_tab[dev_i]) {
+    cudaError_t e = cudaFuncSetAttribute(ge2e_fused_contrast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ct);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ge2e_phase_contrast_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ct);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ge2e_phase_contrast_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ct);
+    if (e != cudaSuccess) { set_error("svb_ge2e: cudaFuncSetAttribute (contrast)", e); return SVB_ERR_CUDA; }
+    max_smem_ct_tab[dev_i] = (int)smem_ct;
+  }
   const int NMr = N * M;
   const int dtl = (D + kTN - 1) / kTN;
   const int b1tiles = ((NMr + kTM - 1) / kTM) * ((Nc + kTN - 1) / kTN);
@@ -982,8 +1175,12 @@ static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int
   const int b2blocks = (NMr + kWarps - 1) / kWarps;
   int want = N;
   if (b1tiles > want) want = b1tiles;
-  if (ctiles > want && a.need_grad) want = ctiles;
+  if (ctiles > want && a.need_grad && !contrast) want = ctiles;
   if (b2blocks > want) want = b2blocks;
+  // contrast phase D with foreign centroids: one block per centroid gathers its P_k
+  const int dblocks_ct = (Cext && a.need_grad && Nc > N) ? Nc : N;
+  const int dgrid = dblocks_ct < 4 * num_sms ? dblocks_ct : 4 * num_sms;
+  if (contrast && dblocks_ct > want) want = dblocks_ct;
   if (fused == 1 && spk_candidate(N, M, D, Nc) && !Cext && w && !dcos && !cos_out && N <= num_sms) {
     // small batch (the reference's training batch): one CTA or one 2-CTA cluster per speaker, three phases
     static int cluster_ok = 1;                       // cleared if the cluster launch is refused
@@ -991,9 +1188,9 @@ static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int
     for (int CL = (cluster_ok && D % 8 == 0 && 2 * N <= num_sms) ? 2 : 1; CL >= 1; --CL) {
       const size_t sm = spk_layout(N, D / CL, MP).floats * sizeof(float);
       if (sm > 220 * 1024) break;
-      void* fn = spk_kernel(MP, CL);
-      static int spk_smem_tab[kMaxDevices][2][kSpkMaxM / 2] = {};
-      int (&spk_smem_set)[2][kSpkMaxM / 2] = spk_smem_tab[dev_i];
+      void* fn = spk_kernel(MP, CL, loss);
+      static int spk_smem_tab[kMaxDevices][2][2][kSpkMaxM / 2] = {};
+      int (&spk_smem_set)[2][kSpkMaxM / 2] = spk_smem_tab[dev_i][contrast ? 1 : 0];
       if ((int)sm > spk_smem_set[CL - 1][MP / 2 - 1]) {
         cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         if (e != cudaSuccess) { set_error("svb_ge2e: cudaFuncSetAttribute (speaker kernel)", e); return SVB_ERR_CUDA; }
@@ -1109,6 +1306,13 @@ static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int
     ge2e_phase_kernel<0><<<N < 4 * num_sms ? N : 4 * num_sms, kThreads, smem, s>>>(a);
     int e = gemm3(a.Eh, a.El, NMr, D, 0, a.Ch, a.Cl, Nc, D, 0, a.cosm, NMr, Nc, D, 1);               // cos = E^ C^T
     if (e) return e;
+    if (contrast) {          // contrast row phase, then phase D's gathers: no A_off split, no R / P products
+      ge2e_phase_contrast_kernel<2><<<b2blocks, kThreads, 0, s>>>(a);
+      ge2e_phase_contrast_kernel<4><<<dgrid, kThreads, smem_ct, s>>>(a);
+      cudaError_t ce = cudaGetLastError();
+      if (ce != cudaSuccess) { set_error("svb_ge2e: launch (tensor-core path, contrast)", ce); return SVB_ERR_CUDA; }
+      return SVB_OK;
+    }
     ge2e_phase_kernel<2><<<b2blocks, kThreads, 0, s>>>(a);
     if (a.need_grad) {
       e = gemm3(a.Ah, a.Al, NMr, Nc, 0, a.Ch, a.Cl, D, D, 1, a.R, NMr, D, Nc, 1);                   // R = A_off C^
@@ -1124,14 +1328,22 @@ static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int
   }
   a.Eh = a.El = a.Ch = a.Cl = a.Ah = a.Al = nullptr;      // (the fp32 paths do not write the splits)
   if (fused) {
+    const void* fk = contrast ? (const void*)ge2e_fused_contrast_kernel : (const void*)ge2e_fused_kernel;
     int per_sm = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ge2e_fused_kernel, kThreads, smem);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fk, kThreads, smem_ct);
     if (per_sm < 1) { set_error("svb_ge2e: kernel does not fit", cudaSuccess); return SVB_ERR_UNSUPPORTED; }
     if (per_sm > 4) per_sm = 4;
     int grid = want < per_sm * num_sms ? want : per_sm * num_sms;
     void* params[] = {&a};
-    cudaError_t e = cudaLaunchCooperativeKernel((void*)ge2e_fused_kernel, dim3(grid), dim3(kThreads), params, smem, s);
+    cudaError_t e = cudaLaunchCooperativeKernel(fk, dim3(grid), dim3(kThreads), params, smem_ct, s);
     if (e != cudaSuccess) { set_error("svb_ge2e: cooperative launch", e); return SVB_ERR_CUDA; }
+  } else if (contrast) {
+    ge2e_phase_kernel<0><<<N, kThreads, smem, s>>>(a);
+    ge2e_phase_kernel<1><<<b1tiles, kThreads, smem, s>>>(a);
+    ge2e_phase_contrast_kernel<2><<<b2blocks, kThreads, 0, s>>>(a);
+    ge2e_phase_contrast_kernel<4><<<dblocks_ct, kThreads, smem_ct, s>>>(a);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { set_error("svb_ge2e: launch", e); return SVB_ERR_CUDA; }
   } else {
     ge2e_phase_kernel<0><<<N, kThreads, smem, s>>>(a);
     ge2e_phase_kernel<1><<<b1tiles, kThreads, smem, s>>>(a);
@@ -1144,12 +1356,19 @@ static int ge2e_impl(const float* E, const float* Cext, int N, int M, int D, int
   return SVB_OK;
 }
 
+extern "C" int svb_ge2e_ex(const float* E, const float* Cext, int N, int M, int D, int Nc, const float* w,
+                           const float* b, const float* dcos, const float* gscale, float* cos_out, float* per_out,
+                           float* loss_out, float* dE, float* dCext, float* dw, float* db, void* workspace,
+                           size_t workspace_bytes, int fused, int loss, void* stream) {
+  return ge2e_impl(E, Cext, N, M, D, Nc, 0, w, b, dcos, gscale, cos_out, per_out, loss_out, dE, dCext, dw, db, workspace,
+                   workspace_bytes, fused, loss, stream);
+}
 extern "C" int svb_ge2e(const float* E, const float* Cext, int N, int M, int D, int Nc, const float* w,
                         const float* b, const float* dcos, const float* gscale, float* cos_out, float* per_out,
                         float* loss_out, float* dE, float* dCext, float* dw, float* db, void* workspace,
                         size_t workspace_bytes, int fused, void* stream) {
-  return ge2e_impl(E, Cext, N, M, D, Nc, 0, w, b, dcos, gscale, cos_out, per_out, loss_out, dE, dCext, dw, db, workspace,
-                   workspace_bytes, fused, stream);
+  return svb_ge2e_ex(E, Cext, N, M, D, Nc, w, b, dcos, gscale, cos_out, per_out, loss_out, dE, dCext, dw, db, workspace,
+                     workspace_bytes, fused, SVB_GE2E_SOFTMAX, stream);
 }
 
 // Row shard of a global GE2E batch (multi-GPU, SURVEY.md section 8e design A): E holds the M utterances of the N_local
@@ -1158,12 +1377,19 @@ extern "C" int svb_ge2e(const float* E, const float* Cext, int N, int M, int D, 
 // cosine (utils.py:91,113).  Outputs: the shard's part of the loss / dw / db (to be summed over the ranks), dE of the
 // shard's rows WITHOUT the path through their own centroid, and dC (Nc, D): this shard's contribution to the gradient
 // of every centroid (summed over the ranks, row j of the total is then spread over speaker j's utterances as dC_j / M).
+extern "C" int svb_ge2e_rows_ex(const float* E, const float* C, int N_local, int M, int D, int Nc, int col0,
+                                const float* w, const float* b, const float* gscale, float* per_out, float* loss_out,
+                                float* dE, float* dC, float* dw, float* db, void* workspace, size_t workspace_bytes,
+                                int loss, void* stream) {
+  if (!C || !w || !b) { set_error("svb_ge2e_rows: centroids, w and b are required", cudaSuccess); return SVB_ERR_ARG; }
+  return ge2e_impl(E, C, N_local, M, D, Nc, col0, w, b, nullptr, gscale, nullptr, per_out, loss_out, dE, dC, dw, db,
+                   workspace, workspace_bytes, 2, loss, stream);
+}
 extern "C" int svb_ge2e_rows(const float* E, const float* C, int N_local, int M, int D, int Nc, int col0, const float* w,
                              const float* b, const float* gscale, float* per_out, float* loss_out, float* dE, float* dC,
                              float* dw, float* db, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!C || !w || !b) { set_error("svb_ge2e_rows: centroids, w and b are required", cudaSuccess); return SVB_ERR_ARG; }
-  return ge2e_impl(E, C, N_local, M, D, Nc, col0, w, b, nullptr, gscale, nullptr, per_out, loss_out, dE, dC, dw, db,
-                   workspace, workspace_bytes, 2, stream);
+  return svb_ge2e_rows_ex(E, C, N_local, M, D, Nc, col0, w, b, gscale, per_out, loss_out, dE, dC, dw, db, workspace,
+                          workspace_bytes, SVB_GE2E_SOFTMAX, stream);
 }
 
 // Sum over the utterance axis in the order torch's CPU sum kernel uses for this layout (reduction over a strided
@@ -1268,6 +1494,29 @@ __global__ void calc_loss_kernel(const float* __restrict__ S, float* __restrict_
     for (int k = lane; k < Nc; k += 32) dS[(size_t)row * Nc + k] = gs * (expf(s[k] - mx) / den - (k == j ? 1.f : 0.f));
   }
 }
+// The contrast loss on a caller-supplied S: per = 1 - sig(S_jj) + sig(S_jk*) (k* = argmax_{k != j} S_jk, lowest index
+// among ties); dS = gscale * G with G_jj = -sig sig(-.), G_jk* = sig sig(-.), zero elsewhere.  One warp per row.
+__global__ void calc_loss_contrast_kernel(const float* __restrict__ S, float* __restrict__ per, float* __restrict__ dS,
+                                          const float* __restrict__ gscale, int N, int M, int Nc) {
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (row >= N * M) return;
+  const int j = row / M;
+  const float* s = S + (size_t)row * Nc;
+  float sk = -INFINITY;
+  int ks = -1;
+  for (int k = lane; k < Nc; k += 32) {
+    if (k == j) continue;
+    if (ks < 0 || s[k] > sk) { sk = s[k]; ks = k; }
+  }
+  warp_argmax(sk, ks);
+  const ContrastRow c = contrast_row(s[j], sk);
+  if (lane == 0) per[row] = c.per;
+  if (dS) {
+    const float gs = gscale ? *gscale : 1.0f;
+    for (int k = lane; k < Nc; k += 32) dS[(size_t)row * Nc + k] = k == j ? gs * c.gd : (k == ks ? gs * c.gk : 0.f);
+  }
+}
 __global__ void sum_kernel(const float* __restrict__ x, float* __restrict__ out, int n) {
   __shared__ float red[8];
   float v = 0.f;
@@ -1275,11 +1524,18 @@ __global__ void sum_kernel(const float* __restrict__ x, float* __restrict__ out,
   v = block_sum(v, red);
   if (threadIdx.x == 0) *out = v;
 }
-extern "C" int svb_calc_loss(const float* S, int N, int M, int Nc, float* per_out, float* loss_out, float* dS,
-                             const float* gscale, void* stream) {
+extern "C" int svb_calc_loss_ex(const float* S, int N, int M, int Nc, float* per_out, float* loss_out, float* dS,
+                                const float* gscale, int loss, void* stream) {
   if (!S || !per_out || N < 1 || M < 1 || Nc < N) return SVB_ERR_ARG;
+  if (loss != kSoftmax && loss != kContrast) { set_error("svb_calc_loss: unknown loss method", cudaSuccess); return SVB_ERR_ARG; }
+  if (loss == kContrast && Nc < 2) { set_error("svb_calc_loss: the contrast loss needs at least two columns", cudaSuccess); return SVB_ERR_ARG; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  calc_loss_kernel<<<(N * M + 7) / 8, 256, 0, st>>>(S, per_out, dS, gscale, N, M, Nc);
+  if (loss == kContrast) calc_loss_contrast_kernel<<<(N * M + 7) / 8, 256, 0, st>>>(S, per_out, dS, gscale, N, M, Nc);
+  else calc_loss_kernel<<<(N * M + 7) / 8, 256, 0, st>>>(S, per_out, dS, gscale, N, M, Nc);
   if (loss_out) sum_kernel<<<1, 256, 0, st>>>(per_out, loss_out, N * M);
   return cudaGetLastError() == cudaSuccess ? SVB_OK : SVB_ERR_CUDA;
+}
+extern "C" int svb_calc_loss(const float* S, int N, int M, int Nc, float* per_out, float* loss_out, float* dS,
+                             const float* gscale, void* stream) {
+  return svb_calc_loss_ex(S, N, M, Nc, per_out, loss_out, dS, gscale, SVB_GE2E_SOFTMAX, stream);
 }

@@ -9,6 +9,8 @@ all-reduced with SUM -- not mean -- because the reference loss is a sum over row
 
 The reference has no distributed code at all; this module is new functionality behind the same GE2ELoss object.
 """
+import functools
+
 import torch
 import torch.distributed as dist
 
@@ -23,13 +25,18 @@ def speaker_shard(n_speakers, rank, world):
     return rank * per, (rank + 1) * per
 
 
-def _fused_loss_and_grads(E, w, b):
-    return torch.ops.svb200.ge2e_loss(E, w, b, 1, True)
+def _fused_loss_and_grads(E, w, b, loss=0):
+    return torch.ops.svb200.ge2e_loss(E, w, b, 1, True, int(loss))
 
 
-def _rows_loss_and_grads(E_local, C_all, w, b, col0):
+def _rows_loss_and_grads(E_local, C_all, w, b, col0, loss=0):
     """-> (reduction buffer [dC (N*D) | loss, dw, db] of this rank's rows, dE of the rows without the centroid path)"""
-    return torch.ops.svb200.ge2e_rows(E_local, C_all, w, b, int(col0))
+    return torch.ops.svb200.ge2e_rows(E_local, C_all, w, b, int(col0), int(loss))
+
+
+def _native_rows(compute_rows):
+    """True for the library's row-shard arithmetic (with or without a bound loss method)."""
+    return compute_rows is _rows_loss_and_grads or getattr(compute_rows, "func", None) is _rows_loss_and_grads
 
 
 class _GlobalGE2EFn(torch.autograd.Function):
@@ -69,7 +76,7 @@ class _ShardedGE2EFn(torch.autograd.Function):
         rank = dist.get_rank(group)
         Nl, M, D = local_emb.shape
         E = local_emb.contiguous()
-        C_local = E.mean(dim=1) if compute_rows is not _rows_loss_and_grads else torch.ops.svb200.centroids(E)
+        C_local = torch.ops.svb200.centroids(E) if _native_rows(compute_rows) else E.mean(dim=1)
         C_all = torch.empty(world * Nl, D, dtype=E.dtype, device=E.device)
         dist.all_gather_into_tensor(C_all, C_local.contiguous(), group=group)
         red, dE = compute_rows(E, C_all, w.detach(), b.detach(), rank * Nl)
@@ -118,14 +125,14 @@ class _PeerGE2EFn(torch.autograd.Function):
     """Design "A" with the exchange over peer memory: same arithmetic as _ShardedGE2EFn, no NCCL call on the GE2E path."""
 
     @staticmethod
-    def forward(ctx, local_emb, w, b, px):
+    def forward(ctx, local_emb, w, b, px, loss=0):
         Nl, M, D = local_emb.shape
         E = local_emb.contiguous()
         N = px.nc
         px.buf[:Nl * D].view(Nl, D).copy_(torch.ops.svb200.centroids(E))
         px.handle.barrier(channel=0)                       # every rank's centroids are in its buffer
         C_all = torch.ops.svb200.peer_gather(px.buf, px.ptrs, px.world, px.off_c, px.len_c)[:, :Nl * D].reshape(N, D)
-        red, dE = torch.ops.svb200.ge2e_rows(E, C_all.contiguous(), w.detach(), b.detach(), px.rank * Nl)
+        red, dE = torch.ops.svb200.ge2e_rows(E, C_all.contiguous(), w.detach(), b.detach(), px.rank * Nl, int(loss))
         px.buf[px.off_red:px.off_red + px.len_red].copy_(red)
         px.handle.barrier(channel=1)                       # every rank's partials are in its buffer
         dC_own, tail = torch.ops.svb200.peer_reduce(px.buf, px.ptrs, px.world, px.off_red, px.rank * Nl * D, Nl * D,
@@ -138,7 +145,7 @@ class _PeerGE2EFn(torch.autograd.Function):
     def backward(ctx, g):
         dE, dw, db = ctx.saved_tensors
         dE, dw, db = torch.ops.svb200.scale3(dE, dw, db, g)
-        return dE, dw, db, None
+        return dE, dw, db, None, None
 
 
 
@@ -151,7 +158,8 @@ class GlobalGE2ELoss(torch.nn.Module):
     centroid gradients (design A); ``mode="peer"``: the same with both exchange steps over NVLink peer memory
     (symmetric buffers, svb_peer_gather / svb_peer_reduce, no NCCL call on the GE2E path; falls back to "rows" where
     symmetric memory is unavailable); ``mode="gather"``: d-vector all-gather, every rank evaluates the global batch
-    (design B, round 1).  ``compute`` injects the arithmetic (host-logic tests on CPU / gloo)."""
+    (design B, round 1).  ``compute`` injects the arithmetic (host-logic tests on CPU / gloo).  Without it, the loss
+    method is the criterion's ``loss_method`` ("softmax" or "contrast"), read at every call."""
 
     def __init__(self, criterion, group=None, compute=None, mode="rows"):
         super().__init__()
@@ -160,8 +168,20 @@ class GlobalGE2ELoss(torch.nn.Module):
         self.criterion = criterion
         self.group = group
         self.mode = mode
+        self._default_compute = compute is None
         self.compute = compute or (_fused_loss_and_grads if mode == "gather" else _rows_loss_and_grads)
         self._px = None
+
+    def _loss_code(self):
+        return ops.loss_code(getattr(self.criterion, "loss_method", "softmax"))
+
+    def _compute(self):
+        """The arithmetic of this call: an injected ``compute`` as given, else the library's with the criterion's loss
+        method bound (the softmax default is the plain function)."""
+        code = self._loss_code()
+        if not self._default_compute or code == 0:
+            return self.compute
+        return functools.partial(self.compute, loss=code)
 
     def _peer(self, E):
         """The symmetric buffers of this (group, shape), or None when peer memory is not available (-> NCCL rows)."""
@@ -184,9 +204,9 @@ class GlobalGE2ELoss(torch.nn.Module):
         if self.mode == "peer" and local_embeddings.is_cuda:
             px = self._peer(local_embeddings)
             if px is not None:
-                return _PeerGE2EFn.apply(local_embeddings, self.criterion.w, self.criterion.b, px)
+                return _PeerGE2EFn.apply(local_embeddings, self.criterion.w, self.criterion.b, px, self._loss_code())
         fn = _GlobalGE2EFn if self.mode == "gather" else _ShardedGE2EFn
-        return fn.apply(local_embeddings, self.criterion.w, self.criterion.b, self.group, self.compute)
+        return fn.apply(local_embeddings, self.criterion.w, self.criterion.b, self.group, self._compute())
 
 
 class PeerAllReduce:

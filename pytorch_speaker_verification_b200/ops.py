@@ -328,7 +328,28 @@ def embedder_forward(x, cache, dims, params):
 
 
 # ------------------------------------------------------------------------------------------ GE2E ops
-def _ge2e_call(E, Cext, w, b, dcos, gscale, want_cos, want_loss, need_grad, fused=1):
+# GE2E loss methods (include/svb200.h SVB_GE2E_*): Wan et al. eq. 6 (the reference's) and eq. 7
+LOSS_METHODS = {"softmax": 0, "contrast": 1}
+
+
+def loss_code(method):
+    """'softmax' / 'contrast' (or their codes 0 / 1) -> the C ABI's SVB_GE2E_* code; anything else raises ValueError."""
+    if isinstance(method, str) and method in LOSS_METHODS:
+        return LOSS_METHODS[method]
+    if not isinstance(method, (str, bool)) and method in LOSS_METHODS.values():
+        return int(method)
+    raise ValueError(f"unknown GE2E loss method {method!r}: expected one of {sorted(LOSS_METHODS)}")
+
+
+def _check_loss(loss, columns):
+    code = loss_code(loss)
+    if code == LOSS_METHODS["contrast"] and columns < 2:
+        raise ValueError("the GE2E contrast loss needs at least 2 centroid columns (speakers): it scores every row "
+                         "against its most similar other centroid")
+    return code
+
+
+def _ge2e_call(E, Cext, w, b, dcos, gscale, want_cos, want_loss, need_grad, fused=1, loss=0):
     N, M, D = (int(s) for s in E.shape)
     Nc = N if Cext is None else int(Cext.shape[0])
     dev = E.device
@@ -339,43 +360,45 @@ def _ge2e_call(E, Cext, w, b, dcos, gscale, want_cos, want_loss, need_grad, fuse
         f32 = dict(dtype=torch.float32, device=dev)
         cos = torch.empty(N, M, Nc, **f32) if want_cos else None
         per = torch.empty(N, M, **f32) if want_loss else None
-        loss = torch.empty((), **f32) if want_loss else None
         dE = torch.empty(N, M, D, **f32) if need_grad else None
         dC = torch.empty(Nc, D, **f32) if (need_grad and Cext is not None) else None
         dw = torch.empty((), **f32) if (need_grad and w is not None) else None
         db = torch.empty((), **f32) if (need_grad and w is not None) else None
-        check(_lib.lib().svb_ge2e(ptr(E), ptr(Cext), N, M, D, Nc, ptr(w), ptr(b), ptr(dcos), ptr(gscale), ptr(cos),
-                                  ptr(per), ptr(loss), ptr(dE), ptr(dC), ptr(dw), ptr(db), ptr(ws), _sz(nbytes.value),
-                                  int(fused), stream_ptr(dev)), "svb_ge2e")
-    return dict(cos=cos, per=per, loss=loss, dE=dE, dC=dC, dw=dw, db=db)
+        lsum = torch.empty((), **f32) if want_loss else None
+        check(_lib.lib().svb_ge2e_ex(ptr(E), ptr(Cext), N, M, D, Nc, ptr(w), ptr(b), ptr(dcos), ptr(gscale), ptr(cos),
+                                     ptr(per), ptr(lsum), ptr(dE), ptr(dC), ptr(dw), ptr(db), ptr(ws), _sz(nbytes.value),
+                                     int(fused), int(loss), stream_ptr(dev)), "svb_ge2e_ex")
+    return dict(cos=cos, per=per, loss=lsum, dE=dE, dC=dC, dw=dw, db=db)
 
 
-def _ge2e_loss(E: torch.Tensor, w: torch.Tensor, b: torch.Tensor, fused: int, need_grad: bool
+def _ge2e_loss(E: torch.Tensor, w: torch.Tensor, b: torch.Tensor, fused: int, need_grad: bool, loss: int = 0
                ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
     if E.shape[1] < 2:
         raise ValueError("GE2E needs at least 2 utterances per speaker (leave-one-out centroid, utils.py:56-57)")
-    r = _ge2e_call(E.contiguous(), None, w.contiguous(), b.contiguous(), None, None, False, True, need_grad, fused)
+    loss = _check_loss(loss, E.shape[0])
+    r = _ge2e_call(E.contiguous(), None, w.contiguous(), b.contiguous(), None, None, False, True, need_grad, fused, loss)
     if not need_grad:
         z = E.new_empty(0)
         return r["loss"], z, z.clone(), z.clone()
     return r["loss"], r["dE"], r["dw"], r["db"]
 
 
-def _ge2e_loss_fake(E, w, b, fused, need_grad):
+def _ge2e_loss_fake(E, w, b, fused, need_grad, loss=0):
     if not need_grad:
         return E.new_empty(()), E.new_empty(0), E.new_empty(0), E.new_empty(0)
     return E.new_empty(()), torch.empty_like(E), E.new_empty(()), E.new_empty(())
 
 
 # forward AND gradients in one fused launch: loss plus d loss / d (E, w, b); autograd scales them by the upstream
-_op("ge2e_loss(Tensor E, Tensor w, Tensor b, int fused, bool need_grad) -> (Tensor, Tensor, Tensor, Tensor)",
+_op("ge2e_loss(Tensor E, Tensor w, Tensor b, int fused, bool need_grad, int loss=0) -> (Tensor, Tensor, Tensor, Tensor)",
     _ge2e_loss, _ge2e_loss_fake)
 
 
-def _ge2e_rows(E: torch.Tensor, C: torch.Tensor, w: torch.Tensor, b: torch.Tensor, col0: int
+def _ge2e_rows(E: torch.Tensor, C: torch.Tensor, w: torch.Tensor, b: torch.Tensor, col0: int, loss: int = 0
                ) -> Tuple[torch.Tensor, torch.Tensor]:
     N, M, D = (int(v) for v in E.shape)
     Nc = int(C.shape[0])
+    loss = _check_loss(loss, Nc)
     dev = E.device
     with torch.cuda.device(dev):
         nbytes = _sz(0)
@@ -386,18 +409,20 @@ def _ge2e_rows(E: torch.Tensor, C: torch.Tensor, w: torch.Tensor, b: torch.Tenso
         dE = torch.empty(N, M, D, dtype=torch.float32, device=dev)
         base = red.data_ptr()
         f = lambda off: ctypes.c_void_p(base + 4 * off)
-        check(_lib.lib().svb_ge2e_rows(ptr(E.contiguous()), ptr(C.contiguous()), N, M, D, Nc, int(col0), ptr(w.contiguous()),
-                                       ptr(b.contiguous()), None, None, f(Nc * D), ptr(dE), f(0), f(Nc * D + 1),
-                                       f(Nc * D + 2), ptr(ws), _sz(nbytes.value), stream_ptr(dev)), "svb_ge2e_rows")
+        check(_lib.lib().svb_ge2e_rows_ex(ptr(E.contiguous()), ptr(C.contiguous()), N, M, D, Nc, int(col0),
+                                          ptr(w.contiguous()), ptr(b.contiguous()), None, None, f(Nc * D), ptr(dE), f(0),
+                                          f(Nc * D + 1), f(Nc * D + 2), ptr(ws), _sz(nbytes.value), int(loss),
+                                          stream_ptr(dev)), "svb_ge2e_rows_ex")
     return red, dE
 
 
-def _ge2e_rows_fake(E, C, w, b, col0):
+def _ge2e_rows_fake(E, C, w, b, col0, loss=0):
     return E.new_empty(C.shape[0] * C.shape[1] + 3), torch.empty_like(E)
 
 
 # row shard of a global batch against all-gathered centroids: (reduction buffer [dC | loss, dw, db], dE of the shard)
-_op("ge2e_rows(Tensor E, Tensor C, Tensor w, Tensor b, int col0) -> (Tensor, Tensor)", _ge2e_rows, _ge2e_rows_fake)
+_op("ge2e_rows(Tensor E, Tensor C, Tensor w, Tensor b, int col0, int loss=0) -> (Tensor, Tensor)", _ge2e_rows,
+    _ge2e_rows_fake)
 
 
 def _peer_gather(anchor: torch.Tensor, peer_ptrs_dev: int, world: int, offset: int, n: int) -> torch.Tensor:
@@ -485,28 +510,30 @@ def _ge2e_setup(ctx, inputs, output):
 
 def _ge2e_backward(ctx, g, *_unused):
     if g is None:
-        return None, None, None, None, None
+        return None, None, None, None, None, None
     if not ctx.need:
         raise RuntimeError("svb200::ge2e_loss was run with need_grad=False")
     dE, dw, db = ctx.saved_tensors
     a, b, c = torch.ops.svb200.scale3(dE, dw, db, g.to(torch.float32))
-    return a, b, c, None, None
+    return a, b, c, None, None, None
 
 
 torch.library.register_autograd(f"{NS}::ge2e_loss", _ge2e_backward, setup_context=_ge2e_setup)
 
 
-def ge2e_loss(E, w, b, fused=1):
-    """GE2ELoss.forward + backward in one fused kernel (speech_embedder_net.py:43-49, utils.py:27-132)."""
+def ge2e_loss(E, w, b, fused=1, loss_method="softmax"):
+    """GE2ELoss.forward + backward in one fused kernel (speech_embedder_net.py:43-49, utils.py:27-132).
+    ``loss_method``: "softmax" (the reference's, Wan et al. eq. 6) or "contrast" (eq. 7)."""
     if E.dim() != 3:
         raise ValueError("embeddings must be (speakers, utterances, dim)")
     if E.shape[1] < 2:
         raise ValueError("GE2E needs at least 2 utterances per speaker (leave-one-out centroid, utils.py:56-57)")
+    code = _check_loss(loss_method, E.shape[0])
     dev = _target_device(E, w, b)
     need = torch.is_grad_enabled() and (E.requires_grad or w.requires_grad or b.requires_grad)
     with torch.cuda.device(dev):
         loss = torch.ops.svb200.ge2e_loss(_stage(E, torch.float32, dev), _stage(w, torch.float32, dev),
-                                          _stage(b, torch.float32, dev), int(fused), bool(need))[0]
+                                          _stage(b, torch.float32, dev), int(fused), bool(need), code)[0]
     return _back(loss, E.device)
 
 
@@ -570,39 +597,47 @@ torch.library.register_autograd(
     setup_context=lambda ctx, inputs, output: ctx.save_for_backward(inputs[0], inputs[1]))
 
 
-def _calc_loss(S: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+def _calc_loss(S: torch.Tensor, loss: int = 0) -> Tuple[torch.Tensor, torch.Tensor]:
     N, M, Nc = (int(s) for s in S.shape)
+    code = _check_loss(loss, Nc)
     S = S.contiguous()
-    per, loss = _f32(S, N, M), _f32(S)
+    per, lsum = _f32(S, N, M), _f32(S)
     with torch.cuda.device(S.device):
-        check(_lib.lib().svb_calc_loss(ptr(S), N, M, Nc, ptr(per), ptr(loss), None, None, stream_ptr(S.device)),
-              "svb_calc_loss")
-    return loss, per
+        check(_lib.lib().svb_calc_loss_ex(ptr(S), N, M, Nc, ptr(per), ptr(lsum), None, None, code, stream_ptr(S.device)),
+              "svb_calc_loss_ex")
+    return lsum, per
 
 
-def _calc_loss_bwd(S: torch.Tensor, gloss: torch.Tensor) -> torch.Tensor:
+def _calc_loss_bwd(S: torch.Tensor, gloss: torch.Tensor, loss: int = 0) -> torch.Tensor:
     N, M, Nc = (int(s) for s in S.shape)
+    code = _check_loss(loss, Nc)
     S = S.contiguous()
     per, dS = _f32(S, N, M), torch.empty_like(S)
     with torch.cuda.device(S.device):
-        check(_lib.lib().svb_calc_loss(ptr(S), N, M, Nc, ptr(per), None, ptr(dS), ptr(gloss.contiguous()),
-                                       stream_ptr(S.device)), "svb_calc_loss")
+        check(_lib.lib().svb_calc_loss_ex(ptr(S), N, M, Nc, ptr(per), None, ptr(dS), ptr(gloss.contiguous()), code,
+                                          stream_ptr(S.device)), "svb_calc_loss_ex")
     return dS
 
 
-_op("calc_loss(Tensor S) -> (Tensor, Tensor)", _calc_loss, lambda S: (S.new_empty(()), S.new_empty(S.shape[0], S.shape[1])))
-_op("calc_loss_bwd(Tensor S, Tensor gloss) -> Tensor", _calc_loss_bwd, lambda S, g: torch.empty_like(S))
+_op("calc_loss(Tensor S, int loss=0) -> (Tensor, Tensor)", _calc_loss,
+    lambda S, loss=0: (S.new_empty(()), S.new_empty(S.shape[0], S.shape[1])))
+_op("calc_loss_bwd(Tensor S, Tensor gloss, int loss=0) -> Tensor", _calc_loss_bwd, lambda S, g, loss=0: torch.empty_like(S))
 
 
 def _calc_loss_setup(ctx, inputs, output):
     ctx.set_materialize_grads(False)
     ctx.save_for_backward(inputs[0])
+    ctx.loss = int(inputs[1]) if len(inputs) > 1 else 0
     ctx.mark_non_differentiable(output[1])       # the reference's per-embedding loss is used for logging only
 
 
-torch.library.register_autograd(
-    f"{NS}::calc_loss", lambda ctx, gloss, _gper: None if gloss is None else torch.ops.svb200.calc_loss_bwd(ctx.saved_tensors[0], gloss.to(torch.float32)),
-    setup_context=_calc_loss_setup)
+def _calc_loss_backward(ctx, gloss, _gper):
+    if gloss is None:
+        return None, None
+    return torch.ops.svb200.calc_loss_bwd(ctx.saved_tensors[0], gloss.to(torch.float32), ctx.loss), None
+
+
+torch.library.register_autograd(f"{NS}::calc_loss", _calc_loss_backward, setup_context=_calc_loss_setup)
 
 
 def get_centroids(E):
@@ -634,12 +669,14 @@ def get_cossim(E, C):
     return _back(torch.ops.svb200.cossim(_stage(E, torch.float32, dev), _stage(C, torch.float32, dev)), E.device)
 
 
-def calc_loss(S):
-    """utils.calc_loss (utils.py:126-132): (loss, per_embedding_loss)."""
+def calc_loss(S, loss_method="softmax"):
+    """utils.calc_loss (utils.py:126-132): (loss, per_embedding_loss); ``loss_method`` "contrast" gives the GE2E
+    contrast loss (Wan et al. eq. 7) of the same similarity matrix."""
     if S.dim() != 3 or S.shape[2] < S.shape[0]:
         raise ValueError("calc_loss expects a similarity matrix (N, M, N)")
+    code = _check_loss(loss_method, S.shape[2])
     dev = _target_device(S)
-    loss, per = torch.ops.svb200.calc_loss(_stage(S, torch.float32, dev))
+    loss, per = torch.ops.svb200.calc_loss(_stage(S, torch.float32, dev), code)
     return _back(loss, S.device), _back(per, S.device)
 
 

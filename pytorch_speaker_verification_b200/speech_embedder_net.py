@@ -51,15 +51,19 @@ class SpeechEmbedder(nn.Module):
 
 
 class GE2ELoss(nn.Module):
-    """GE2E softmax loss with learnable w, b (speech_embedder_net.py:35-49)."""
+    """GE2E loss with learnable w, b (speech_embedder_net.py:35-49).  ``loss_method``: "softmax" (default, the
+    reference's loss, Wan et al. eq. 6) or "contrast" (eq. 7: 1 - sigmoid(S_jj) + sigmoid of the most similar other
+    centroid, summed over the embeddings).  Like ``fused``, it is a plain attribute: ``state_dict`` holds w and b only."""
 
-    def __init__(self, device):
+    def __init__(self, device, loss_method="softmax"):
         super(GE2ELoss, self).__init__()
+        ops.loss_code(loss_method)                       # ValueError for an unknown method
         self.w = nn.Parameter(torch.tensor(10.0).to(device), requires_grad=True)
         self.b = nn.Parameter(torch.tensor(-5.0).to(device), requires_grad=True)
         self.device = device
         self.fused = True
+        self.loss_method = loss_method
 
     def forward(self, embeddings):
         # speech_embedder_net.py:44 `torch.clamp(self.w, 1e-6)` discards its result: w is NOT clamped.
-        return ops.ge2e_loss(embeddings, self.w, self.b, int(self.fused))
+        return ops.ge2e_loss(embeddings, self.w, self.b, int(self.fused), self.loss_method)

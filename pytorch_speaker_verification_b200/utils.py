@@ -24,6 +24,7 @@ def get_cossim(embeddings, centroids):
     return ops.get_cossim(embeddings, centroids)
 
 
-def calc_loss(sim_matrix):
-    """(N, M, N) -> (loss, per_embedding_loss (N, M)); loss is the SUM over rows (utils.py:126-132)."""
-    return ops.calc_loss(sim_matrix)
+def calc_loss(sim_matrix, loss_method="softmax"):
+    """(N, M, N) -> (loss, per_embedding_loss (N, M)); loss is the SUM over rows (utils.py:126-132).
+    ``loss_method="contrast"``: the GE2E contrast loss (Wan et al. eq. 7) instead of the softmax loss (eq. 6)."""
+    return ops.calc_loss(sim_matrix, loss_method)
