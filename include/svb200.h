@@ -229,6 +229,28 @@ int svb_eer_finish(const int* cnt_all, const int* cnt_diag, int N, int Mv, int T
 int svb_eer_sweep(const float* sim, int N, int Mv, const float* thresholds, int T, int* cnt_all, int* cnt_diag,
                   unsigned long long* scratch, float* out, void* stream);
 
+/* ---- exact EER and minDCF over every score threshold (new; DESIGN.md 4.5) ----------------------------------------
+ * Operating point k of the K distinct scores v_1 < ... < v_K accepts the scores >= v_{k+1} (point K accepts nothing,
+ * threshold +inf).  EER: the point with the smallest |miss * Nn - fa * Nt| (exact integers, ties to the smaller k),
+ * reported as (p_miss + p_fa) / 2.  minDCF of each operating point (w_miss, w_fa, c_def): the smallest
+ * (w_miss * p_miss + w_fa * p_fa) / c_def, every float64 operation rounded separately, ties to the smaller k.  -0.0 counts
+ * as +0.0.  Bit-exact and run-to-run identical.  2 <= n < 2^31.
+ * The workspace (about 18.04 n bytes) holds two 8n-byte element buffers, the radix sort's per-tile digit count / offset
+ * table (8 KB per 4096 scores, rewritten by every pass), a counter region that every call clears (cudaMemsetAsync on
+ * `stream`: 24 KB plus 4 B per 4096 scores) and the sweep's per-tile results (148 B per 4096 scores).  No allocation
+ * and no host synchronisation, so the calls can be captured in a CUDA graph. */
+int svb_verif_workspace_bytes(int64_t n, size_t* bytes);
+/* ops: HOST array of 3*P doubles {w_miss, w_fa, c_def} per operating point, 1 <= P <= 8.
+ * out (device, 8 + 4P doubles): eer, eer threshold, eer p_miss, eer p_fa, Nt, Nn, #non-finite scores, K,
+ * then per point: min_dcf, threshold, p_miss, p_fa.  With a non-finite score or an empty class the metrics are NaN.
+ * labels: n bytes, nonzero = target. */
+int svb_verif_metrics(const float* scores, const uint8_t* labels, int64_t n, const double* ops, int P,
+                      void* workspace, size_t workspace_bytes, double* out, void* stream);
+/* The same for a TI-SV similarity matrix sim (N, Mv, N) (svb_eer_sweep's input): element [j, m, k] is a target trial
+ * iff k == j, the pooled trials behind the reference's FAR and FRR.  n = N * Mv * N, N >= 2. */
+int svb_verif_metrics_sim(const float* sim, int N, int Mv, const double* ops, int P,
+                          void* workspace, size_t workspace_bytes, double* out, void* stream);
+
 /* ---- d-vector extraction (dvector_create.py:48-52,98-99 and :55-73) ----------------------------------------------- */
 
 /* Sliding windows of a (nmels, Ttot) log-mel matrix (row pitch ldS) -> (W, win, nmels); win_start (W) int32 device. */

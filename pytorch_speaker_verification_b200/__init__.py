@@ -6,6 +6,8 @@ backed by hand-written CUDA kernels behind the C ABI in include/svb200.h.  No CP
 from .speech_embedder_net import GE2ELoss, SpeechEmbedder            # noqa: F401
 from .utils import calc_loss, get_centroids, get_cossim              # noqa: F401
 from .eer import compute_eer, eer_sweep                              # noqa: F401
+from .eer import (VerificationMetrics, compute_verification_metrics,  # noqa: F401
+                  verification_metrics, verification_metrics_from_sim)
 from .dvector import align_embeddings, extract_dvectors, get_windows  # noqa: F401
 from .optim import FusedClipSGD                                       # noqa: F401
 from .staging import prefetch                                         # noqa: F401

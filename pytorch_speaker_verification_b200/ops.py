@@ -746,6 +746,55 @@ def eer_finish(cnt_all, cnt_diag, Mv):
     return torch.ops.svb200.eer_finish(cnt_all, cnt_diag, int(Mv))
 
 
+# ------------------------------------------------------------------------------------------ exact EER / minDCF ops
+# out (8 + 4P float64): eer, threshold, p_miss, p_fa, Nt, Nn, #non-finite, K, then per point min_dcf, threshold,
+# p_miss, p_fa (include/svb200.h svb_verif_metrics)
+def _verif_call(fn, what, n, args, ops, dev):
+    P = len(ops) // 3
+    with torch.cuda.device(dev):
+        nbytes = _sz(0)
+        check(_lib.lib().svb_verif_workspace_bytes(_i64(n), ctypes.byref(nbytes)), "svb_verif_workspace_bytes")
+        ws = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+        out = torch.empty(8 + 4 * P, dtype=torch.float64, device=dev)
+        check(fn(*args, (ctypes.c_double * len(ops))(*ops), P, ptr(ws), _sz(nbytes.value), ptr(out), stream_ptr(dev)),
+              what)
+    return out
+
+
+def _verif_metrics(scores: torch.Tensor, labels: torch.Tensor, ops: List[float]) -> torch.Tensor:
+    if scores.dtype != torch.float32 or labels.dtype not in (torch.uint8, torch.bool) or scores.shape != labels.shape:
+        raise ValueError("verif_metrics expects float32 scores and uint8 / bool labels of the same shape")
+    if labels.device != scores.device:
+        raise ValueError(f"verif_metrics: labels on {labels.device}, scores on {scores.device}: they must share the "
+                         "CUDA device")
+    s, lab = scores.contiguous(), labels.contiguous()
+    n = s.numel()
+    return _verif_call(_lib.lib().svb_verif_metrics, "svb_verif_metrics", n, (ptr(s), ptr(lab), _i64(n)), ops, s.device)
+
+
+def _verif_metrics_sim(sim: torch.Tensor, ops: List[float]) -> torch.Tensor:
+    if sim.dtype != torch.float32 or sim.dim() != 3 or sim.shape[0] != sim.shape[2]:
+        raise ValueError("verif_metrics_sim expects a float32 similarity matrix (N, Mv, N)")
+    s = sim.contiguous()
+    N, Mv = int(s.shape[0]), int(s.shape[1])
+    return _verif_call(_lib.lib().svb_verif_metrics_sim, "svb_verif_metrics_sim", N * Mv * N, (ptr(s), N, Mv), ops,
+                       s.device)
+
+
+_op("verif_metrics(Tensor scores, Tensor labels, float[] ops) -> Tensor", _verif_metrics,
+    lambda scores, labels, ops: scores.new_empty(8 + 4 * (len(ops) // 3), dtype=torch.float64))
+_op("verif_metrics_sim(Tensor sim, float[] ops) -> Tensor", _verif_metrics_sim,
+    lambda sim, ops: sim.new_empty(8 + 4 * (len(ops) // 3), dtype=torch.float64))
+
+
+def verif_metrics(scores, labels_u8, ops):
+    return torch.ops.svb200.verif_metrics(scores, labels_u8, [float(v) for v in ops])
+
+
+def verif_metrics_sim(sim, ops):
+    return torch.ops.svb200.verif_metrics_sim(sim, [float(v) for v in ops])
+
+
 # ------------------------------------------------------------------------------------------ d-vector ops
 def _dvector_windows(S: torch.Tensor, win_start: torch.Tensor, win: int) -> torch.Tensor:
     nmels, W = int(S.shape[0]), int(win_start.numel())
@@ -820,4 +869,4 @@ _op("logmel(Tensor y, Tensor window, Tensor twiddle, Tensor mel_w, int hop, int 
 
 OP_NAMES = ["pack_weights", "embedder_fwd", "embedder_bwd", "ge2e_loss", "ge2e_rows", "scale3", "centroids", "centroids_bwd",
             "utterance_centroids", "cossim", "cossim_bwd", "calc_loss", "calc_loss_bwd", "eer_counts", "eer_sweep", "peer_gather", "peer_reduce",
-            "eer_finish", "dvector_windows", "segment_mean", "clip_sgd", "logmel"]
+            "eer_finish", "verif_metrics", "verif_metrics_sim", "dvector_windows", "segment_mean", "clip_sgd", "logmel"]
