@@ -50,8 +50,9 @@ def init_state_dict(nmels=40, hidden=768, num_layer=3, proj=256, seed=0):
 
 @dataclass
 class Emu:
-    """Which operands are rounded to bf16 (hi) or to a hi+lo bf16 pair ("split")."""
-    x_in: str = "fp32"      # activations entering the input-projection GEMM: fp32|bf16|split
+    """Which operands are rounded to bf16 (hi), to a hi+lo bf16 pair ("split") or to fp16 (the operand format of the
+    forward GEMMs)."""
+    x_in: str = "fp32"      # activations entering the input-projection GEMM: fp32|bf16|split|fp16
     w_in: str = "fp32"      # W_ih
     h_rec: str = "fp32"     # h_{t-1} entering the recurrent GEMM
     w_rec: str = "fp32"     # W_hh
@@ -61,6 +62,8 @@ class Emu:
 def _rnd(t, mode):
     if mode == "fp32":
         return t
+    if mode == "fp16":
+        return t.to(torch.float16).to(t.dtype)
     hi = t.to(torch.bfloat16).to(t.dtype)
     if mode == "bf16":
         return hi

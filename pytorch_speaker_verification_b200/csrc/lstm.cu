@@ -733,7 +733,8 @@ static void prof_mark(int phase, cudaStream_t s) {   // phase >= 0: start of a p
 #define SVB_CUDA(what) do { cudaError_t _e = cudaGetLastError(); if (_e != cudaSuccess) { set_error(what, _e); return SVB_ERR_CUDA; } } while (0)
 
 static int check_dims(const Dims& d) {
-  if (d.B < 1 || d.T < 1 || d.I < 1 || d.L < 1 || d.L > 8 || d.P < 1) { set_error("embedder: bad dims", cudaSuccess); return SVB_ERR_ARG; }
+  if (d.L < 1 || d.L > 8) { set_error("embedder: num_layer must be 1 to 8", cudaSuccess); return SVB_ERR_ARG; }
+  if (d.B < 1 || d.T < 1 || d.I < 1 || d.P < 1) { set_error("embedder: batch, frames, nmels and proj must be positive", cudaSuccess); return SVB_ERR_ARG; }
   if (d.H % 128 != 0) { set_error("embedder: hidden size must be a multiple of 128", cudaSuccess); return SVB_ERR_UNSUPPORTED; }
   return SVB_OK;
 }
@@ -844,7 +845,10 @@ extern "C" int svb_embedder_forward(const void* x, int x_dtype, const void* pack
     if (training) cudaMemsetAsync(w.gates[l] + (size_t)T * B * 4 * H, 0, (size_t)B * 4 * H * 2, s);
   }
   bool use_wlstm = false;
-  if (g_persistent && rec_terms == 1 && L <= 3 && (H == 768 || H == 512 || H == 256)) {
+  // (layer 0's input-projection CTAs keep W_ih resident in tensor memory, 32 columns per 64-wide K block, below the
+  //  accumulators at kWlAccCol: nmels up to 768.  Wider inputs take the per-frame path, which has no such limit.)
+  if (g_persistent && rec_terms == 1 && L <= 3 && (H == 768 || H == 512 || H == 256) &&
+      (Ip0 + 63) / 64 * 32 <= kWlAccCol) {
     const int num_sms = device_sm_count();
     use_wlstm = 2 * L * (H / 32) <= num_sms;
   }

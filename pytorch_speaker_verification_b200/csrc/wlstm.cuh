@@ -25,6 +25,7 @@
 // back-pressure) hcnt[l][j] >= NS*(t-D+1).  The dependency graph is acyclic in (t, l) and all CTAs are co-resident
 // (cooperative launch), so the layers form a self-timed wavefront: layer l runs frame t while layer l+1 runs t-1.
 // TMEM map (512 columns): [0, K/2) = weights, two fp16 per column; [384, 448) and [448, 512) = two accumulators.
+// So K <= 768 (in 64-wide blocks): H <= 768, and nmels <= 768 for layer 0 (svb_embedder_forward checks it).
 #pragma once
 
 constexpr int kWlTile = 64;            // batch rows per tile (= MMA N)
@@ -725,6 +726,11 @@ __global__ void __launch_bounds__(kWlThreads, 1) wlstm_fwd_kernel(const __grid_c
 template <int H>
 static int launch_wlstm_fwd(WlstmParams& p, cudaStream_t s) {
   auto kern = wlstm_fwd_kernel<H>;
+  for (int l = 0; l < p.L; ++l)                    // a wider W_ih slice would overlap the accumulators
+    if ((p.layer[l].Ip + 63) / 64 * 32 > kWlAccCol) {
+      set_error("wlstm: layer input wider than 768 does not fit tensor memory", cudaSuccess);
+      return SVB_ERR_UNSUPPORTED;
+    }
   static unsigned long long configured = 0;        // one bit per device
   if (first_use_on_device(configured)) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kWlSmem);
