@@ -251,6 +251,37 @@ int svb_verif_metrics(const float* scores, const uint8_t* labels, int64_t n, con
 int svb_verif_metrics_sim(const float* sim, int N, int Mv, const double* ops, int P,
                           void* workspace, size_t workspace_bytes, double* out, void* stream);
 
+/* ---- cohort score normalization: S-norm and adaptive S-norm (new; DESIGN.md 4.5.2) --------------------------------
+ * cos(x, y) = (x / |x|) . (y / |y|); a row with a zero or non-finite norm makes every score and statistic it takes part
+ * in NaN.  Cohort statistics of a row x against a cohort C of Nc rows with top-K (2 <= K <= Nc; K = Nc is plain S-norm):
+ * S_K(x) = the multiset of the K largest cos(x, c), mu = mean of S_K(x), sigma = sample standard deviation of S_K(x)
+ * (divisor K - 1), v_K = the K-th largest value.  -0.0 counts as +0.0; a non-finite cohort score makes the row's three
+ * statistics NaN.  Statistics are accumulated and returned in float64 (fixed reduction order, no float atomics:
+ * run-to-run identical).  Normalized score of a trial (e, t) with raw score s:
+ *   s' = 1/2 ((s - mu(e)) / sigma(e) + (s - mu(t)) / sigma(t)),  returned as float32.
+ * No allocation and no host synchronisation, so every call can be captured in a CUDA graph. */
+
+/* Workspace of svb_cohort_stats: the cohort's and one chunk's fp16 hi / lo splits (zero-padded to round64(D) columns,
+ * the cohort to a multiple of 8 rows) and the chunk's fp32 score slab (about 48 MB).  1 <= n < 2^31, 2 <= Nc <= 2^20,
+ * 1 <= D <= 65536. */
+int svb_cohort_stats_workspace_bytes(int64_t n, int Nc, int D, size_t* bytes);
+/* X (n, D), cohort (Nc, D) float32 row-major -> out (n, 3) float64: mu, sigma, v_K.  2 <= K <= Nc.  Cohort cosines are
+ * 3-term split-fp16 tensor-core products (about 2^-22 relative); the workspace is 256-byte aligned. */
+int svb_cohort_stats(const float* X, int64_t n, const float* cohort, int Nc, int D, int K, void* workspace,
+                     size_t workspace_bytes, double* out, void* stream);
+/* The same statistics of caller-supplied cohort scores: row i is scores[i * ld, i * ld + Nc).  ld >= Nc. */
+int svb_cohort_stats_scores(const float* scores, int64_t n, int Nc, int64_t ld, int K, double* out, void* stream);
+/* out[i] = cos(E[ei[i]], T[ti[i]]) for E (ne, D), T (nt, D), int32 indices (validated by the caller: an index out of
+ * range gives NaN and reads nothing); with stats_e (ne, 3) and stats_t (nt, 3) from svb_cohort_stats the normalized
+ * score instead.  stats_e and stats_t are both NULL (raw cosine) or both given. */
+int svb_score_trials(const float* E, int64_t ne, const float* T, int64_t nt, int D, const int32_t* ei,
+                     const int32_t* ti, int64_t n_trials, const double* stats_e, const double* stats_t, float* out,
+                     void* stream);
+/* TI-SV matrix sim (N, Mv, N) (svb_verif_metrics_sim's input): out[j, m, k] = the normalized score of sim[j, m, k] with
+ * stats_c (N, 3) of the enrollment centroids k and stats_v (N * Mv, 3) of the verification utterances [j, m]. */
+int svb_asnorm_sim(const float* sim, int N, int Mv, const double* stats_c, const double* stats_v, float* out,
+                   void* stream);
+
 /* ---- d-vector extraction (dvector_create.py:48-52,98-99 and :55-73) ----------------------------------------------- */
 
 /* Sliding windows of a (nmels, Ttot) log-mel matrix (row pitch ldS) -> (W, win, nmels); win_start (W) int32 device. */

@@ -7,6 +7,7 @@ import numbers
 import torch
 
 from . import ops
+from .scoring import normalize_sim
 from .utils import get_centroids, get_cossim
 
 THRESHOLDS = [0.01 * i + 0.5 for i in range(50)]          # train_speech_embedder.py:134
@@ -141,8 +142,13 @@ def verification_metrics_from_sim(sim_matrix, p_target=0.01, c_miss=1.0, c_fa=1.
     return _metrics_from_out(out, len(ops_) // 3)
 
 
-def compute_verification_metrics(enrollment_embeddings, verification_embeddings, p_target=0.01, c_miss=1.0, c_fa=1.0):
-    """compute_eer's similarity matrix scored exactly: (VerificationMetrics, sim_matrix)."""
+def compute_verification_metrics(enrollment_embeddings, verification_embeddings, p_target=0.01, c_miss=1.0, c_fa=1.0,
+                                 *, cohort=None, top_k=None):
+    """compute_eer's similarity matrix scored exactly: (VerificationMetrics, sim_matrix).  With a ``cohort`` (Nc, D) of
+    impostor embeddings the matrix is first S-norm (top_k None) or AS-norm normalized (scoring.normalize_sim), and the
+    normalized matrix is returned."""
     enrollment_centroids = get_centroids(enrollment_embeddings)
     sim_matrix = get_cossim(verification_embeddings, enrollment_centroids)
+    if cohort is not None:
+        sim_matrix = normalize_sim(sim_matrix, enrollment_centroids, verification_embeddings, cohort, top_k)
     return verification_metrics_from_sim(sim_matrix, p_target, c_miss, c_fa), sim_matrix

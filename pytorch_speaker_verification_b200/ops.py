@@ -795,6 +795,116 @@ def verif_metrics_sim(sim, ops):
     return torch.ops.svb200.verif_metrics_sim(sim, [float(v) for v in ops])
 
 
+# ------------------------------------------------------------------------------------------ cohort score normalization
+# statistics (n, 3) float64: mean, std (divisor K - 1), K-th largest cohort score (include/svb200.h svb_cohort_stats)
+def _same_device(what, *tensors):
+    for t in tensors:
+        if t is not None and t.device != tensors[0].device:
+            raise ValueError(f"{what}: tensors on {tensors[0].device} and {t.device}: they must share the CUDA device")
+
+
+def _cohort_stats(X: torch.Tensor, cohort: torch.Tensor, top_k: int) -> torch.Tensor:
+    if (X.dtype != torch.float32 or cohort.dtype != torch.float32 or X.dim() != 2 or cohort.dim() != 2
+            or X.shape[1] != cohort.shape[1]):
+        raise ValueError("cohort_stats expects float32 rows (n, D) and a float32 cohort (Nc, D)")
+    _same_device("cohort_stats", X, cohort)
+    x, c = X.contiguous(), cohort.contiguous()
+    n, D, Nc = int(x.shape[0]), int(x.shape[1]), int(c.shape[0])
+    out = torch.empty(n, 3, dtype=torch.float64, device=x.device)
+    if n == 0:
+        return out
+    with torch.cuda.device(x.device):
+        nbytes = _sz(0)
+        check(_lib.lib().svb_cohort_stats_workspace_bytes(_i64(n), Nc, D, ctypes.byref(nbytes)),
+              "svb_cohort_stats_workspace_bytes")
+        ws = torch.empty(nbytes.value, dtype=torch.uint8, device=x.device)
+        check(_lib.lib().svb_cohort_stats(ptr(x), _i64(n), ptr(c), Nc, D, int(top_k), ptr(ws), _sz(nbytes.value),
+                                          ptr(out), stream_ptr(x.device)), "svb_cohort_stats")
+    return out
+
+
+def _cohort_stats_scores(scores: torch.Tensor, top_k: int) -> torch.Tensor:
+    if scores.dtype != torch.float32 or scores.dim() != 2:
+        raise ValueError("cohort_stats_scores expects float32 cohort scores (n, Nc)")
+    s = scores if scores.stride(1) == 1 and scores.stride(0) >= scores.shape[1] else scores.contiguous()
+    n, Nc = int(s.shape[0]), int(s.shape[1])
+    out = torch.empty(n, 3, dtype=torch.float64, device=s.device)
+    if n == 0:
+        return out
+    with torch.cuda.device(s.device):
+        check(_lib.lib().svb_cohort_stats_scores(ptr(s), _i64(n), Nc, _i64(s.stride(0)), int(top_k), ptr(out),
+                                                 stream_ptr(s.device)), "svb_cohort_stats_scores")
+    return out
+
+
+def _score_trials(E: torch.Tensor, T: torch.Tensor, ei: torch.Tensor, ti: torch.Tensor,
+                  stats_e: Optional[torch.Tensor], stats_t: Optional[torch.Tensor]) -> torch.Tensor:
+    if (E.dtype != torch.float32 or T.dtype != torch.float32 or E.dim() != 2 or T.dim() != 2
+            or E.shape[1] != T.shape[1]):
+        raise ValueError("score_trials expects float32 rows E (ne, D) and T (nt, D)")
+    if ei.dtype != torch.int32 or ti.dtype != torch.int32 or ei.shape != ti.shape or ei.dim() != 1:
+        raise ValueError("score_trials expects int32 index vectors of one length")
+    if (stats_e is None) != (stats_t is None):
+        raise ValueError("score_trials: give the statistics of both sides or of neither")
+    if stats_e is not None and (stats_e.dtype != torch.float64 or stats_t.dtype != torch.float64
+                                or tuple(stats_e.shape) != (E.shape[0], 3) or tuple(stats_t.shape) != (T.shape[0], 3)):
+        raise ValueError("score_trials expects float64 statistics (ne, 3) and (nt, 3)")
+    _same_device("score_trials", E, T, ei, ti, stats_e, stats_t)
+    e, t, a, b = E.contiguous(), T.contiguous(), ei.contiguous(), ti.contiguous()
+    se = None if stats_e is None else stats_e.contiguous()
+    st = None if stats_t is None else stats_t.contiguous()
+    out = torch.empty(a.numel(), dtype=torch.float32, device=e.device)
+    with torch.cuda.device(e.device):
+        check(_lib.lib().svb_score_trials(ptr(e), _i64(e.shape[0]), ptr(t), _i64(t.shape[0]), int(e.shape[1]), ptr(a),
+                                          ptr(b), _i64(a.numel()), ptr(se), ptr(st), ptr(out), stream_ptr(e.device)),
+              "svb_score_trials")
+    return out
+
+
+def _asnorm_sim(sim: torch.Tensor, stats_c: torch.Tensor, stats_v: torch.Tensor) -> torch.Tensor:
+    if sim.dtype != torch.float32 or sim.dim() != 3 or sim.shape[0] != sim.shape[2]:
+        raise ValueError("asnorm_sim expects a float32 similarity matrix (N, Mv, N)")
+    N, Mv = int(sim.shape[0]), int(sim.shape[1])
+    if (stats_c.dtype != torch.float64 or stats_v.dtype != torch.float64 or tuple(stats_c.shape) != (N, 3)
+            or tuple(stats_v.shape) != (N * Mv, 3)):
+        raise ValueError("asnorm_sim expects float64 statistics (N, 3) and (N * Mv, 3)")
+    _same_device("asnorm_sim", sim, stats_c, stats_v)
+    s = sim.contiguous()
+    out = torch.empty_like(s)
+    if s.numel() == 0:
+        return out
+    with torch.cuda.device(s.device):
+        check(_lib.lib().svb_asnorm_sim(ptr(s), N, Mv, ptr(stats_c.contiguous()), ptr(stats_v.contiguous()), ptr(out),
+                                        stream_ptr(s.device)), "svb_asnorm_sim")
+    return out
+
+
+_op("cohort_stats(Tensor X, Tensor cohort, int top_k) -> Tensor", _cohort_stats,
+    lambda X, cohort, top_k: X.new_empty(X.shape[0], 3, dtype=torch.float64))
+_op("cohort_stats_scores(Tensor scores, int top_k) -> Tensor", _cohort_stats_scores,
+    lambda scores, top_k: scores.new_empty(scores.shape[0], 3, dtype=torch.float64))
+_op("score_trials(Tensor E, Tensor T, Tensor ei, Tensor ti, Tensor? stats_e, Tensor? stats_t) -> Tensor", _score_trials,
+    lambda E, T, ei, ti, stats_e, stats_t: E.new_empty(ei.shape[0], dtype=torch.float32))
+_op("asnorm_sim(Tensor sim, Tensor stats_c, Tensor stats_v) -> Tensor", _asnorm_sim,
+    lambda sim, stats_c, stats_v: torch.empty_like(sim))
+
+
+def cohort_stats(X, cohort, top_k):
+    return torch.ops.svb200.cohort_stats(X, cohort, int(top_k))
+
+
+def cohort_stats_scores(scores, top_k):
+    return torch.ops.svb200.cohort_stats_scores(scores, int(top_k))
+
+
+def score_trials(E, T, ei, ti, stats_e=None, stats_t=None):
+    return torch.ops.svb200.score_trials(E, T, ei, ti, stats_e, stats_t)
+
+
+def asnorm_sim(sim, stats_c, stats_v):
+    return torch.ops.svb200.asnorm_sim(sim, stats_c, stats_v)
+
+
 # ------------------------------------------------------------------------------------------ d-vector ops
 def _dvector_windows(S: torch.Tensor, win_start: torch.Tensor, win: int) -> torch.Tensor:
     nmels, W = int(S.shape[0]), int(win_start.numel())
@@ -869,4 +979,5 @@ _op("logmel(Tensor y, Tensor window, Tensor twiddle, Tensor mel_w, int hop, int 
 
 OP_NAMES = ["pack_weights", "embedder_fwd", "embedder_bwd", "ge2e_loss", "ge2e_rows", "scale3", "centroids", "centroids_bwd",
             "utterance_centroids", "cossim", "cossim_bwd", "calc_loss", "calc_loss_bwd", "eer_counts", "eer_sweep", "peer_gather", "peer_reduce",
-            "eer_finish", "verif_metrics", "verif_metrics_sim", "dvector_windows", "segment_mean", "clip_sgd", "logmel"]
+            "eer_finish", "verif_metrics", "verif_metrics_sim", "cohort_stats", "cohort_stats_scores", "score_trials",
+            "asnorm_sim", "dvector_windows", "segment_mean", "clip_sgd", "logmel"]
