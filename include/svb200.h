@@ -251,6 +251,47 @@ int svb_verif_metrics(const float* scores, const uint8_t* labels, int64_t n, con
 int svb_verif_metrics_sim(const float* sim, int N, int Mv, const double* ops, int P,
                           void* workspace, size_t workspace_bytes, double* out, void* stream);
 
+/* ---- score calibration and calibration metrics (new; DESIGN.md 4.5.3) ---------------------------------------------
+ * Scores are float32 natural-log likelihood ratios l; Nt / Nn are the target / non-target counts.  -0.0 counts as +0.0,
+ * denormals stay distinct; a non-finite score makes every metric NaN.
+ *   Cllr = 1/2 [ (1/Nt) sum_tar softplus(-l) + (1/Nn) sum_non softplus(l) ] / ln 2,  softplus(x) = log(1 + e^x).
+ *   Actual DCF of an operating point (w_miss, w_fa, c_def) (as svb_verif_metrics takes them): threshold
+ *   theta = log(w_fa / w_miss) (host float64); a trial is accepted iff (double)l >= theta; miss = targets below theta,
+ *   fa = non-targets at or above it; act_dcf = (w_miss * miss/Nt + w_fa * fa/Nn) / c_def, every float64 operation
+ *   rounded separately.
+ *   minCllr: the Cllr after the optimal non-decreasing map from score to LLR (PAV, tied scores pooled).  With the
+ *   cumulative points (X_g, Y_g) = (trials, targets in the groups of equal scores up to g), from (0, 0), it is read off
+ *   their lower convex hull: a hull segment of m trials, t targets and f = m - t non-targets adds t log2(1 + f Nt/(t Nn))
+ *   to the target sum and f log2(1 + t Nn/(f Nt)) to the non-target sum (a term with a zero count adds 0), and
+ *   minCllr = 1/2 (target sum / Nt + non-target sum / Nn).  Hull tests are exact int64 cross products; collinear points
+ *   are dropped.
+ *   ROCCH-EER: the hull vertices as ROC points (P_miss = Y/Nt, P_fa = (Nn - (X - Y))/Nn); the value e where that
+ *   polyline crosses P_miss = P_fa, in float64.
+ *   Linear calibration at prior pi, tau = logit(pi): (a, b) minimises
+ *   C(a, b) = (pi/Nt) sum_tar softplus(-(a s + b + tau)) + ((1 - pi)/Nn) sum_non softplus(a s + b + tau).  A finite,
+ *   unique minimiser exists iff min_tar < max_non and min_non < max_tar.  At pi = 1/2, C / ln 2 is the Cllr of a s + b.
+ * Float64 sums in a fixed order, no float atomics: run-to-run and stream-to-stream identical.  No allocation and no host
+ * synchronisation, so both calls can be captured in a CUDA graph.  2 <= n < 2^31.
+ * The workspace (about 18.04 n bytes, 256-byte aligned) serves both calls: svb_verif_metrics' sort buffers (the first
+ * holds the convex hulls once the sort is done), 12 B per 4096 scores of hull bookkeeping, per-block partials. */
+#define SVB_CALIB_CONVERGED 0
+#define SVB_CALIB_SEPARABLE 1          /* the classes do not overlap strictly (includes fewer than two distinct scores) */
+#define SVB_CALIB_ITERATION_CAP 2      /* max_iter passes without convergence */
+#define SVB_CALIB_BAD_INPUT 3          /* an empty class or a non-finite score */
+int svb_calib_workspace_bytes(int64_t n, size_t* bytes);
+/* ops: HOST array of 3*P doubles {w_miss, w_fa, c_def}, 1 <= P <= 8.  out (device, 8 + 4P doubles): cllr, min_cllr,
+ * rocch_eer, Nt, Nn, #non-finite scores, #hull vertices (with the origin), K (distinct scores), then per point:
+ * act_dcf, theta, p_miss, p_fa.  labels: n bytes, nonzero = target. */
+int svb_calib_metrics(const float* llr, const uint8_t* labels, int64_t n, const double* ops, int P,
+                      void* workspace, size_t workspace_bytes, double* out, void* stream);
+/* Damped Newton from (a, b) = (0, 0): one fused pass over the scores (objective, gradient, Hessian) and a one-block
+ * update per iteration, max_iter >= 1 of them enqueued; it stops when half the squared Newton decrement is <= 1e-12
+ * (then takes that last step without a line search).  0 < prior < 1.  out (device, 5 doubles): a, b, C(a, b) / ln 2,
+ * iterations (objective evaluations), status (SVB_CALIB_*); a, b and C are NaN unless the status is CONVERGED or
+ * ITERATION_CAP. */
+int svb_calib_train(const float* scores, const uint8_t* labels, int64_t n, double prior, int max_iter,
+                    void* workspace, size_t workspace_bytes, double* out, void* stream);
+
 /* ---- cohort score normalization: S-norm and adaptive S-norm (new; DESIGN.md 4.5.2) --------------------------------
  * cos(x, y) = (x / |x|) . (y / |y|); a row with a zero or non-finite norm makes every score and statistic it takes part
  * in NaN.  Cohort statistics of a row x against a cohort C of Nc rows with top-K (2 <= K <= Nc; K = Nc is plain S-norm):

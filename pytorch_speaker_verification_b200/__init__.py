@@ -9,6 +9,8 @@ from .eer import compute_eer, eer_sweep                              # noqa: F40
 from .eer import (VerificationMetrics, compute_verification_metrics,  # noqa: F401
                   verification_metrics, verification_metrics_from_sim)
 from .scoring import cohort_stats, normalize_sim, score_trials        # noqa: F401
+from .calibration import (Calibration, CalibrationMetrics,             # noqa: F401
+                          apply_calibration, calibration_metrics, train_calibration)
 from .dvector import align_embeddings, extract_dvectors, get_windows  # noqa: F401
 from .optim import FusedClipSGD                                       # noqa: F401
 from .staging import prefetch                                         # noqa: F401

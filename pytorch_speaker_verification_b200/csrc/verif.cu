@@ -15,6 +15,7 @@
 // allocate nor synchronise, so a CUDA graph can capture them.  DESIGN.md 4.5.1 explains why the sort is not onesweep.
 #include "../../include/svb200.h"
 #include "perdev.cuh"
+#include "verif_sort.cuh"
 #include <cuda_runtime.h>
 #include <math.h>
 #include <algorithm>
@@ -24,17 +25,10 @@ namespace svb {
 void set_error(const char* what, cudaError_t e);
 
 namespace verif {
-constexpr int kDigitBits = 11;
-constexpr int kBins = 1 << kDigitBits;                 // 2048
-constexpr int kPasses = 3;                             // 33-bit elements
 constexpr int kMaxPoints = 8;
 
 constexpr int kKeyThreads = 512;
 
-constexpr int kSortThreads = 256;
-constexpr int kSortWarps = kSortThreads / 32;
-constexpr int kSortItems = 16;                         // per thread
-constexpr int kSortTile = kSortThreads * kSortItems;   // 4096 elements
 constexpr int kBinsPerThread = kBins / kSortThreads;   // 8
 
 constexpr int kSweepThreads = 256;
@@ -59,18 +53,6 @@ struct Best {
 
 __device__ __forceinline__ bool better(const Best& a, const Best& b) {
   return a.v < b.v || (a.v == b.v && a.pos < b.pos);
-}
-
-__device__ __forceinline__ uint32_t score_key(float x, unsigned& nonfinite) {
-  uint32_t u = __float_as_uint(x);
-  if (u == 0x80000000u) u = 0u;                        // -0 counts as +0 (bit test: denormals stay distinct)
-  nonfinite += (u & 0x7f800000u) == 0x7f800000u;
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
-__device__ __forceinline__ double key_value(uint32_t key) {
-  const uint32_t u = (key & 0x80000000u) ? (key & 0x7fffffffu) : ~key;
-  return (double)__uint_as_float(u);
 }
 
 __device__ __forceinline__ uint32_t digit_of(unsigned long long e, int shift) {
@@ -167,31 +149,6 @@ __global__ void __launch_bounds__(kKeyThreads) verif_key_kernel(const float* __r
   }
   for (int b = threadIdx.x; b < kPasses * kBins; b += blockDim.x)
     if (h[b]) atomicAdd(&ghist[b], h[b]);
-}
-
-// ------------------------------------------------------------------------------------------ block scans (256 threads)
-// Exclusive scan of one value per thread over the block; returns the prefix, *total = the block's sum.
-template <int kThreads>
-__device__ __forceinline__ uint32_t block_excl_scan(uint32_t v, uint32_t* warp_tot, uint32_t* total) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t incl = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const uint32_t y = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += y;
-  }
-  if (lane == 31) warp_tot[warp] = incl;
-  __syncthreads();
-  uint32_t before = 0, all = 0;
-#pragma unroll
-  for (int w = 0; w < kThreads / 32; ++w) {
-    const uint32_t t = warp_tot[w];
-    before += w < warp ? t : 0u;
-    all += t;
-  }
-  __syncthreads();                                     // warp_tot may be reused by the caller's next scan
-  *total = all;
-  return before + incl - v;
 }
 
 // ------------------------------------------------------------------------------------- (b) sort passes
@@ -623,6 +580,29 @@ inline Layout layout(int64_t n) {
 
 inline bool n_ok(int64_t n) { return n >= 2 && n < (int64_t(1) << 31); }
 
+// After three passes (A -> B -> A -> B) the sorted elements are in B.
+cudaError_t sort_elements(const float* scores, const uint8_t* labels, int n, int N, int MvN, const SortBuffers& sb,
+                          cudaStream_t st) {
+  static unsigned long long attr_done = 0;
+  if (first_use_on_device(attr_done)) {
+    const cudaError_t e = cudaFuncSetAttribute(verif_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               (int)sizeof(SortSmem));
+    if (e != cudaSuccess) { attr_done = 0; return e; }
+  }
+  const int tiles = sort_tiles(n);
+  const int key_blocks = (int)std::min<int64_t>(2 * device_sm_count(), ((int64_t)n + 4 * kKeyThreads - 1) / (4 * kKeyThreads));
+  verif_key_kernel<<<std::max(key_blocks, 1), kKeyThreads, 0, st>>>(scores, labels, n, N, MvN, sb.a, sb.hist, sb.counts);
+  unsigned long long* src = sb.a;
+  unsigned long long* dst = sb.b;
+  for (int p = 0; p < kPasses; ++p) {
+    verif_count_kernel<<<tiles, kSortThreads, 0, st>>>(src, n, p * kDigitBits, sb.offs);
+    verif_scan_kernel<<<kBins / kScanDigits, kSortThreads, 0, st>>>(sb.offs, tiles, sb.hist + p * kBins);
+    verif_scatter_kernel<<<tiles, kSortThreads, sizeof(SortSmem), st>>>(src, dst, n, p * kDigitBits, sb.offs);
+    std::swap(src, dst);
+  }
+  return cudaGetLastError();
+}
+
 int run(const float* scores, const uint8_t* labels, int64_t n64, int N, int MvN, const double* ops, int P,
         void* workspace, size_t workspace_bytes, double* out, void* stream, const char* who) {
   if (!scores || !ops || !workspace || !out || !n_ok(n64) || P < 1 || P > kMaxPoints) {
@@ -648,32 +628,19 @@ int run(const float* scores, const uint8_t* labels, int64_t n64, int N, int MvN,
   }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   char* ws = static_cast<char*>(workspace);
-  auto* A = reinterpret_cast<unsigned long long*>(ws + L.a);
-  auto* B = reinterpret_cast<unsigned long long*>(ws + L.b);
-  auto* hist = reinterpret_cast<uint32_t*>(ws + L.hist);
-  auto* counts = reinterpret_cast<unsigned long long*>(ws + L.counts);
+  SortBuffers sb;
+  sb.a = reinterpret_cast<unsigned long long*>(ws + L.a);
+  sb.b = reinterpret_cast<unsigned long long*>(ws + L.b);
+  sb.offs = reinterpret_cast<uint32_t*>(ws + L.offs);
+  sb.hist = reinterpret_cast<uint32_t*>(ws + L.hist);
+  sb.counts = reinterpret_cast<unsigned long long*>(ws + L.counts);
   auto* tickets = reinterpret_cast<unsigned*>(ws + L.tickets);
-  auto* offs = reinterpret_cast<uint32_t*>(ws + L.offs);
   auto* sweep_status = reinterpret_cast<uint32_t*>(ws + L.sweep_status);
 
   cudaError_t e = cudaMemsetAsync(ws + L.ctr, 0, L.ctr_bytes, st);
+  if (e == cudaSuccess) e = sort_elements(scores, labels, n, N, MvN, sb, st);
   if (e != cudaSuccess) { set_error(who, e); return SVB_ERR_CUDA; }
-  static unsigned long long attr_done = 0;
-  if (first_use_on_device(attr_done)) {
-    e = cudaFuncSetAttribute(verif_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SortSmem));
-    if (e != cudaSuccess) { attr_done = 0; set_error(who, e); return SVB_ERR_CUDA; }
-  }
-  const int key_blocks = (int)std::min<int64_t>(2 * device_sm_count(), (n64 + 4 * kKeyThreads - 1) / (4 * kKeyThreads));
-  verif_key_kernel<<<std::max(key_blocks, 1), kKeyThreads, 0, st>>>(scores, labels, n, N, MvN, A, hist, counts);
-  unsigned long long* src = A;
-  unsigned long long* dst = B;
-  for (int p = 0; p < kPasses; ++p) {
-    verif_count_kernel<<<L.sort_tiles, kSortThreads, 0, st>>>(src, n, p * kDigitBits, offs);
-    verif_scan_kernel<<<kBins / kScanDigits, kSortThreads, 0, st>>>(offs, L.sort_tiles, hist + p * kBins);
-    verif_scatter_kernel<<<L.sort_tiles, kSortThreads, sizeof(SortSmem), st>>>(src, dst, n, p * kDigitBits, offs);
-    std::swap(src, dst);
-  }
-  verif_sweep_kernel<<<L.sweep_tiles, kSweepThreads, 0, st>>>(src, n, counts, sweep_status, tickets,
+  verif_sweep_kernel<<<L.sweep_tiles, kSweepThreads, 0, st>>>(sb.b, n, sb.counts, sweep_status, tickets,
                                                               reinterpret_cast<Best*>(ws + L.best),
                                                               reinterpret_cast<uint32_t*>(ws + L.groups), pt, out);
   e = cudaGetLastError();

@@ -795,6 +795,54 @@ def verif_metrics_sim(sim, ops):
     return torch.ops.svb200.verif_metrics_sim(sim, [float(v) for v in ops])
 
 
+# ------------------------------------------------------------------------------------------ score calibration
+# metrics out (8 + 4P float64): cllr, min_cllr, rocch_eer, Nt, Nn, #non-finite, #hull vertices, K, then per point
+# act_dcf, threshold, p_miss, p_fa; train out (5 float64): a, b, C / ln 2, iterations, status (include/svb200.h)
+def _calib_args(what, scores, labels):
+    if scores.dtype != torch.float32 or labels.dtype not in (torch.uint8, torch.bool) or scores.shape != labels.shape:
+        raise ValueError(f"{what} expects float32 scores and uint8 / bool labels of the same shape")
+    _same_device(what, scores, labels)
+    s, lab = scores.contiguous(), labels.contiguous()
+    n = s.numel()
+    nbytes = _sz(0)
+    with torch.cuda.device(s.device):
+        check(_lib.lib().svb_calib_workspace_bytes(_i64(n), ctypes.byref(nbytes)), "svb_calib_workspace_bytes")
+    return s, lab, n, torch.empty(nbytes.value, dtype=torch.uint8, device=s.device), nbytes.value
+
+
+def _calib_metrics(llr: torch.Tensor, labels: torch.Tensor, ops: List[float]) -> torch.Tensor:
+    s, lab, n, ws, nbytes = _calib_args("calib_metrics", llr, labels)
+    P = len(ops) // 3
+    out = torch.empty(8 + 4 * P, dtype=torch.float64, device=s.device)
+    with torch.cuda.device(s.device):
+        check(_lib.lib().svb_calib_metrics(ptr(s), ptr(lab), _i64(n), (ctypes.c_double * len(ops))(*ops), P, ptr(ws),
+                                           _sz(nbytes), ptr(out), stream_ptr(s.device)), "svb_calib_metrics")
+    return out
+
+
+def _calib_train(scores: torch.Tensor, labels: torch.Tensor, prior: float, max_iter: int) -> torch.Tensor:
+    s, lab, n, ws, nbytes = _calib_args("calib_train", scores, labels)
+    out = torch.empty(5, dtype=torch.float64, device=s.device)
+    with torch.cuda.device(s.device):
+        check(_lib.lib().svb_calib_train(ptr(s), ptr(lab), _i64(n), ctypes.c_double(prior), int(max_iter), ptr(ws),
+                                         _sz(nbytes), ptr(out), stream_ptr(s.device)), "svb_calib_train")
+    return out
+
+
+_op("calib_metrics(Tensor llr, Tensor labels, float[] ops) -> Tensor", _calib_metrics,
+    lambda llr, labels, ops: llr.new_empty(8 + 4 * (len(ops) // 3), dtype=torch.float64))
+_op("calib_train(Tensor scores, Tensor labels, float prior, int max_iter) -> Tensor", _calib_train,
+    lambda scores, labels, prior, max_iter: scores.new_empty(5, dtype=torch.float64))
+
+
+def calib_metrics(llr, labels_u8, ops):
+    return torch.ops.svb200.calib_metrics(llr, labels_u8, [float(v) for v in ops])
+
+
+def calib_train(scores, labels_u8, prior, max_iter):
+    return torch.ops.svb200.calib_train(scores, labels_u8, float(prior), int(max_iter))
+
+
 # ------------------------------------------------------------------------------------------ cohort score normalization
 # statistics (n, 3) float64: mean, std (divisor K - 1), K-th largest cohort score (include/svb200.h svb_cohort_stats)
 def _same_device(what, *tensors):
@@ -980,4 +1028,4 @@ _op("logmel(Tensor y, Tensor window, Tensor twiddle, Tensor mel_w, int hop, int 
 OP_NAMES = ["pack_weights", "embedder_fwd", "embedder_bwd", "ge2e_loss", "ge2e_rows", "scale3", "centroids", "centroids_bwd",
             "utterance_centroids", "cossim", "cossim_bwd", "calc_loss", "calc_loss_bwd", "eer_counts", "eer_sweep", "peer_gather", "peer_reduce",
             "eer_finish", "verif_metrics", "verif_metrics_sim", "cohort_stats", "cohort_stats_scores", "score_trials",
-            "asnorm_sim", "dvector_windows", "segment_mean", "clip_sgd", "logmel"]
+            "asnorm_sim", "calib_metrics", "calib_train", "dvector_windows", "segment_mean", "clip_sgd", "logmel"]
