@@ -28,12 +28,18 @@ const char* svb_last_error(void);
 /* Generic tensor-core GEMM used by the LSTM: C[M,N] = sum_t A_t[M,K] * B_t[N,K]^T (+ bias[n]).
  * bf16 operands, fp32 accumulate/out.  a_mn/b_mn = 1 when the operand is stored [K, rows] instead of [rows, K].
  * A and B are HOST arrays of nterms DEVICE pointers (nterms <= 3). Replaces the aten::addmm / cuDNN GEMMs that
- * nn.LSTM / nn.Linear issue for speech_embedder_net.py:28,31. */
+ * nn.LSTM / nn.Linear issue for speech_embedder_net.py:28,31.
+ * Preconditions, checked before any CUDA call:
+ *   SVB_ERR_ARG unless M, N, K >= 1; 1 <= nterms <= 3; A, B and every A[t], B[t] and C are non-null;
+ *     lda >= K (A K-major) or lda >= M (a_mn); ldb >= K (B K-major) or ldb >= N (b_mn); ldc >= N.
+ *   SVB_ERR_ALIGN unless every A[t], B[t] is 16-byte aligned and lda, ldb are multiples of 8 elements.
+ * C and bias need only float alignment: when C, bias or ldc is not 16-byte aligned, or N % 4 != 0, the epilogue
+ * stores directly instead of through TMA.  Elements of C outside [0, M) x [0, N) are never written. */
 int svb_gemm_bf16(const void* const* A, const void* const* B, int nterms, float* C, const float* bias, int M, int N,
                   int K, int64_t lda, int64_t ldb, int64_t ldc, int a_mn, int b_mn, void* stream);
 
-/* Same contract computed by CTA pairs (tcgen05.mma.cta_group::2, 256 x 256 pair tiles); mn = 0: both operands
- * K-major, mn = 1: both MN-major. */
+/* Same contract and preconditions computed by CTA pairs (tcgen05.mma.cta_group::2, 256 x 256 pair tiles); mn = 0:
+ * both operands K-major, mn = 1: both MN-major (a_mn = b_mn = mn above). */
 int svb_gemm_bf16_2cta(const void* const* A, const void* const* B, int nterms, float* C, const float* bias, int M,
                        int N, int K, int64_t lda, int64_t ldb, int64_t ldc, int mn, void* stream);
 
@@ -41,7 +47,12 @@ int svb_gemm_bf16_2cta(const void* const* A, const void* const* B, int nterms, f
  * batched GEMM, speech_embedder_net.py:19,28: [T*B x 768] . [768 x 3072] at BASELINE configs[1]): C[M,N] (fp32, pitch
  * ldc) = A[M,K] . B[N,K]^T + bias[n].  Operands K-major with 2-byte elements (f16 != 0: IEEE half, else bf16);
  * K % 64 == 0, N % 256 == 0.  74 CTA pairs walk the 256 x 256 tiles; two TMEM accumulators overlap each tile's
- * epilogue with the next tile's MMAs (csrc/pgemm.cu). */
+ * epilogue with the next tile's MMAs (csrc/pgemm.cu).
+ * Preconditions, checked before any CUDA call:
+ *   SVB_ERR_ARG unless A, B, C are non-null; M >= 1; N a positive multiple of 256; K a positive multiple of 64;
+ *     lda >= K; ldb >= K; ldc >= N and a multiple of 4; bias null or 16-byte aligned.
+ *   SVB_ERR_ALIGN unless A, B and C are 16-byte aligned and lda, ldb are multiples of 8 elements.
+ * Elements of C outside [0, M) x [0, N) are never written. */
 int svb_gemm_persistent(const void* A, const void* B, float* C, const float* bias, int M, int N, int K, int64_t lda,
                         int64_t ldb, int64_t ldc, int f16, void* stream);
 

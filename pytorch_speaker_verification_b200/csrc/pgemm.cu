@@ -172,19 +172,31 @@ using namespace svb;
 // K-major, 2-byte elements (f16 != 0: IEEE half, else bf16); K % 64 == 0, N % 256 == 0, 16-byte aligned pitches.
 extern "C" int svb_gemm_persistent(const void* A, const void* B, float* C, const float* bias, int M, int N, int K,
                                    int64_t lda, int64_t ldb, int64_t ldc, int f16, void* stream) {
-  if (!A || !B || !C || M < 1 || N < 256 || N % 256 || K < 64 || K % 64 || (ldc % 4) ||
-      (bias && (reinterpret_cast<uintptr_t>(bias) & 15))) {
-    set_error("svb_gemm_persistent: needs K % 64 == 0, N % 256 == 0, aligned pitches", cudaSuccess);
-    return SVB_ERR_ARG;
-  }
+  const char* fn = "svb_gemm_persistent";
+  if (!A) return host_error(SVB_ERR_ARG, fn, "A is NULL");
+  if (!B) return host_error(SVB_ERR_ARG, fn, "B is NULL");
+  if (!C) return host_error(SVB_ERR_ARG, fn, "C is NULL");
+  if (M < 1) return host_error(SVB_ERR_ARG, fn, "M = %d, needs M >= 1", M);
+  if (N < 256 || N % 256) return host_error(SVB_ERR_ARG, fn, "N = %d, needs a positive multiple of 256", N);
+  if (K < 64 || K % 64) return host_error(SVB_ERR_ARG, fn, "K = %d, needs a positive multiple of 64", K);
+  if (lda < K) return host_error(SVB_ERR_ARG, fn, "lda = %lld, needs lda >= K", (long long)lda);
+  if (ldb < K) return host_error(SVB_ERR_ARG, fn, "ldb = %lld, needs ldb >= K", (long long)ldb);
+  if (ldc < N) return host_error(SVB_ERR_ARG, fn, "ldc = %lld, needs ldc >= N", (long long)ldc);
+  if (ldc % 4) return host_error(SVB_ERR_ARG, fn, "ldc = %lld is not a multiple of 4", (long long)ldc);
+  if (bias && (reinterpret_cast<uintptr_t>(bias) & 15)) return host_error(SVB_ERR_ARG, fn, "bias is not 16-byte aligned");
+  if (lda % 8) return host_error(SVB_ERR_ALIGN, fn, "lda = %lld is not a multiple of 8 elements", (long long)lda);
+  if (ldb % 8) return host_error(SVB_ERR_ALIGN, fn, "ldb = %lld is not a multiple of 8 elements", (long long)ldb);
+  if (reinterpret_cast<uintptr_t>(A) & 15) return host_error(SVB_ERR_ALIGN, fn, "A is not 16-byte aligned");
+  if (reinterpret_cast<uintptr_t>(B) & 15) return host_error(SVB_ERR_ALIGN, fn, "B is not 16-byte aligned");
+  if (reinterpret_cast<uintptr_t>(C) & 15) return host_error(SVB_ERR_ALIGN, fn, "C is not 16-byte aligned");
   PgParams p;
   memset(&p, 0, sizeof(p));
   int e = make_tmap_bf16(&p.ta, A, (uint64_t)K, (uint64_t)M, 1, (uint64_t)lda, (uint64_t)lda * M, kBM);
-  if (e) return e;
+  if (e) return host_error(e, fn, "tensor map of A rejected");
   e = make_tmap_bf16(&p.tb, B, (uint64_t)K, (uint64_t)N, 1, (uint64_t)ldb, (uint64_t)ldb * N, kBM);
-  if (e) return e;
+  if (e) return host_error(e, fn, "tensor map of B rejected");
   e = make_tmap(&p.tc, C, 4, (uint64_t)N, (uint64_t)M, 1, (uint64_t)ldc, (uint64_t)ldc * M, 32, 128, 3);
-  if (e) return e;
+  if (e) return host_error(e, fn, "tensor map of C rejected");
   p.bias = bias; p.M = M; p.N = N; p.K = K; p.f16 = f16;
   static unsigned long long configured = 0;
   if (first_use_on_device(configured)) {

@@ -342,6 +342,8 @@ int make_tmap(CUtensorMap* out, const void* base, int elem_bytes, uint64_t d0, u
 // bf16 operand tile map: box = {64, box_rows, 1}, 128B swizzle.
 int make_tmap_bf16(CUtensorMap* out, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t stride1_elems,
                    uint64_t stride2_elems, uint32_t box_rows);
+// Records "<fn>: <printf-formatted message>" for svb_last_error() and returns `code`.
+int host_error(int code, const char* fn, const char* fmt, ...);
 
 template <int BN, int kStages, bool A_MN, bool B_MN, class Epi, int kEpiWarps = 4, int KSPLIT = 1, bool TWO_CTA = false>
 cudaError_t launch_tc_gemm(const GemmOperands& ops, const typename Epi::Params& ep, cudaStream_t stream) {

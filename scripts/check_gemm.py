@@ -1,8 +1,9 @@
-"""GPU dev check: tcgen05 GEMM core (all operand-layout variants) against torch fp32 matmul of the same
-bf16-rounded operands.  Prints one line per case; exit code 1 if any case is wrong."""
+"""GPU dev timing: the tcgen05 GEMM core (svb_gemm_bf16, one CTA per 128 x 128 tile, and svb_gemm_bf16_2cta, CTA
+pairs on 256 x 256 tiles) on the LSTM input-projection shape (B*T = 102400, 4H = 3072, K = 768), 1 and 3 terms, next
+to cuBLAS.  Correctness is tests/test_gpu_gemm_core.py.  `python scripts/check_gemm.py 2cta` times the pair kernel
+only."""
 import ctypes
 import sys
-import time
 
 import torch
 
@@ -11,138 +12,38 @@ from pytorch_speaker_verification_b200 import _lib
 
 L = _lib.lib()
 dev = torch.device("cuda:0")
-bad = 0
+M, N, K = 102400, 3072, 768
+A = torch.randn(M, K, device=dev).to(torch.bfloat16)
+B = torch.randn(N, K, device=dev).to(torch.bfloat16)
+C = torch.empty(M, N, device=dev)
+i64 = ctypes.c_int64
 
 
-def run(M, N, K, a_mn, b_mn, nterms, bias=False, seed=0):
-    g = torch.Generator(device="cpu").manual_seed(seed)
-    As = [torch.randn(M, K, generator=g).to(dev).to(torch.bfloat16) for _ in range(nterms)]
-    Bs = [torch.randn(N, K, generator=g).to(dev).to(torch.bfloat16) for _ in range(nterms)]
-    bia = torch.randn(N, generator=g).to(dev) if bias else None
-    ref = sum(a.float() @ b.float().t() for a, b in zip(As, Bs))
-    if bias:
-        ref = ref + bia
-    Am = [a.t().contiguous() if a_mn else a.contiguous() for a in As]
-    Bm = [b.t().contiguous() if b_mn else b.contiguous() for b in Bs]
-    lda = M if a_mn else K
-    ldb = N if b_mn else K
-    C = torch.full((M, N), float("nan"), device=dev)
-    PA = (ctypes.c_void_p * nterms)(*[a.data_ptr() for a in Am])
-    PB = (ctypes.c_void_p * nterms)(*[b.data_ptr() for b in Bm])
-    rc = L.svb_gemm_bf16(PA, PB, nterms, _lib.ptr(C), _lib.ptr(bia), M, N, K, ctypes.c_int64(lda),
-                         ctypes.c_int64(ldb), ctypes.c_int64(N), int(a_mn), int(b_mn), _lib.stream_ptr())
+def timed(fn, n=5):
+    for _ in range(2):
+        fn()
     torch.cuda.synchronize()
-    err = (C - ref).abs().max().item()
-    scale = ref.abs().max().item()
-    ok = rc == 0 and err <= 2e-3 * scale + 1e-3 and not torch.isnan(C).any().item()
-    print(f"M={M} N={N} K={K} a_mn={a_mn} b_mn={b_mn} terms={nterms} bias={bias}: rc={rc} maxerr={err:.3e} "
-          f"scale={scale:.2e} {'OK' if ok else 'WRONG'}", flush=True)
-    return ok
-
-
-def run2(M, N, K, nterms, bias=False, seed=0, mn=0):
-    g = torch.Generator(device="cpu").manual_seed(seed)
-    As = [torch.randn(M, K, generator=g).to(dev).to(torch.bfloat16) for _ in range(nterms)]
-    Bs = [torch.randn(N, K, generator=g).to(dev).to(torch.bfloat16) for _ in range(nterms)]
-    bia = torch.randn(N, generator=g).to(dev) if bias else None
-    ref = sum(a.float() @ b.float().t() for a, b in zip(As, Bs))
-    if bias:
-        ref = ref + bia
-    C = torch.full((M, N), float("nan"), device=dev)
-    Am = [a.t().contiguous() if mn else a for a in As]
-    Bm = [b.t().contiguous() if mn else b for b in Bs]
-    PA = (ctypes.c_void_p * nterms)(*[a.data_ptr() for a in Am])
-    PB = (ctypes.c_void_p * nterms)(*[b.data_ptr() for b in Bm])
-    rc = L.svb_gemm_bf16_2cta(PA, PB, nterms, _lib.ptr(C), _lib.ptr(bia), M, N, K, ctypes.c_int64(M if mn else K),
-                              ctypes.c_int64(N if mn else K), ctypes.c_int64(N), mn, _lib.stream_ptr())
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(n):
+        fn()
+    e1.record()
     torch.cuda.synchronize()
-    err = (C - ref).abs().max().item()
-    scale = ref.abs().max().item()
-    ok = rc == 0 and err <= 2e-3 * scale + 1e-3 and not torch.isnan(C).any().item()
-    print(f"2CTA mn={mn} M={M} N={N} K={K} terms={nterms} bias={bias}: rc={rc} maxerr={err:.3e} scale={scale:.2e} "
-          f"{'OK' if ok else 'WRONG'}", flush=True)
-    return ok
+    return e0.elapsed_time(e1) / n
 
 
-if len(sys.argv) > 1 and sys.argv[1] == "2cta":
-    bad = 0
-    for c in [(256, 256, 64, 1), (256, 256, 768, 1), (640, 3072, 768, 1), (3600, 3072, 768, 3), (300, 512, 200, 2),
-              (128, 256, 128, 1)]:
-        if not run2(*c, bias=(c[0] % 3 == 0)):
-            bad += 1
-    for c in [(256, 256, 64, 1), (512, 256, 3600, 1), (3072, 768, 3600, 1)]:
-        if not run2(*c, mn=1):
-            bad += 1
-    if bad == 0:
-        M, N, K = 102400, 3072, 768
-        A = torch.randn(M, K, device=dev).to(torch.bfloat16)
-        B = torch.randn(N, K, device=dev).to(torch.bfloat16)
-        C = torch.empty(M, N, device=dev)
-        for nt in (1, 3):
-            PA = (ctypes.c_void_p * nt)(*[A.data_ptr()] * nt)
-            PB = (ctypes.c_void_p * nt)(*[B.data_ptr()] * nt)
-            for fn, name in ((L.svb_gemm_bf16_2cta, "2cta 256x256"),):
-                for _ in range(2):
-                    fn(PA, PB, nt, _lib.ptr(C), None, M, N, K, ctypes.c_int64(K), ctypes.c_int64(K), ctypes.c_int64(N),
-                       0, _lib.stream_ptr())
-                torch.cuda.synchronize()
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record()
-                for _ in range(5):
-                    fn(PA, PB, nt, _lib.ptr(C), None, M, N, K, ctypes.c_int64(K), ctypes.c_int64(K), ctypes.c_int64(N),
-                       0, _lib.stream_ptr())
-                e1.record()
-                torch.cuda.synchronize()
-                ms = e0.elapsed_time(e1) / 5
-                print(f"{name} terms={nt}: {ms:.3f} ms, {2 * M * N * K * nt / ms / 1e9:.1f} TFLOP/s", flush=True)
-    print("BAD", bad)
-    sys.exit(1 if bad else 0)
-
-cases = [
-    (128, 128, 64, 0, 0, 1), (128, 128, 128, 0, 0, 1), (256, 256, 768, 0, 0, 1), (640, 3072, 768, 0, 0, 1),
-    (20, 3072, 40, 0, 0, 1), (20, 3072, 40, 0, 0, 3), (300, 256, 200, 0, 0, 2), (3600, 3072, 768, 0, 0, 3),
-    (128, 128, 64, 1, 1, 1), (256, 128, 128, 1, 1, 1), (3072, 768, 3600, 1, 1, 1), (3072, 40, 3600, 1, 1, 1),
-    (128, 128, 64, 0, 1, 1), (128, 128, 64, 1, 0, 1), (640, 768, 3072, 0, 1, 1),
-]
-for c in cases:
-    try:
-        if not run(*c, bias=(c[0] % 3 == 0)):
-            bad += 1
-    except Exception as e:  # noqa
-        print("EXC", c, e)
-        bad += 1
-        break
-
-# throughput of the input-projection shape (B*T=102400, 4H=3072, K=768)
-if bad == 0:
-    M, N, K = 102400, 3072, 768
-    A = torch.randn(M, K, device=dev).to(torch.bfloat16)
-    B = torch.randn(N, K, device=dev).to(torch.bfloat16)
-    C = torch.empty(M, N, device=dev)
+entries = [("2cta 256x256", lambda PA, PB, nt: L.svb_gemm_bf16_2cta(PA, PB, nt, _lib.ptr(C), None, M, N, K, i64(K), i64(K),
+                                                                     i64(N), 0, _lib.stream_ptr()))]
+if not (len(sys.argv) > 1 and sys.argv[1] == "2cta"):
+    entries.insert(0, ("input-proj GEMM", lambda PA, PB, nt: L.svb_gemm_bf16(PA, PB, nt, _lib.ptr(C), None, M, N, K,
+                                                                             i64(K), i64(K), i64(N), 0, 0,
+                                                                             _lib.stream_ptr())))
+for name, fn in entries:
     for nt in (1, 3):
         PA = (ctypes.c_void_p * nt)(*[A.data_ptr()] * nt)
         PB = (ctypes.c_void_p * nt)(*[B.data_ptr()] * nt)
-        for _ in range(2):
-            L.svb_gemm_bf16(PA, PB, nt, _lib.ptr(C), None, M, N, K, ctypes.c_int64(K), ctypes.c_int64(K),
-                            ctypes.c_int64(N), 0, 0, _lib.stream_ptr())
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(5):
-            L.svb_gemm_bf16(PA, PB, nt, _lib.ptr(C), None, M, N, K, ctypes.c_int64(K), ctypes.c_int64(K),
-                            ctypes.c_int64(N), 0, 0, _lib.stream_ptr())
-        e1.record()
-        torch.cuda.synchronize()
-        ms = e0.elapsed_time(e1) / 5
-        print(f"input-proj GEMM terms={nt}: {ms:.3f} ms, {2 * M * N * K * nt / ms / 1e9:.1f} TFLOP/s", flush=True)
-    t0 = time.time()
-    Cb = (A @ B.t())
-    torch.cuda.synchronize()
-    e0.record()
-    for _ in range(5):
-        Cb = A @ B.t()
-    e1.record()
-    torch.cuda.synchronize()
-    print(f"cuBLAS bf16 same shape: {e0.elapsed_time(e1) / 5:.3f} ms")
-print("BAD", bad)
-sys.exit(1 if bad else 0)
+        assert fn(PA, PB, nt) == 0, L.svb_last_error()
+        ms = timed(lambda: fn(PA, PB, nt))
+        print(f"{name} terms={nt}: {ms:.3f} ms, {2 * M * N * K * nt / ms / 1e9:.1f} TFLOP/s", flush=True)
+if len(entries) == 2:
+    print(f"cuBLAS bf16 same shape: {timed(lambda: A @ B.t()):.3f} ms")

@@ -1,5 +1,5 @@
-"""Dev: persistent CTA-pair GEMM (csrc/pgemm.cu) against torch on bf16/fp16-rounded operands, and its time on the
-LSTM input-projection shape next to the one-tile-per-CTA pair kernel."""
+"""Dev timing: the persistent CTA-pair GEMM (csrc/pgemm.cu) on the LSTM input-projection shape next to the
+one-tile-per-CTA pair kernel.  Correctness is tests/test_gpu_gemm_core.py."""
 import ctypes, sys
 import torch
 sys.path.insert(0, "."); sys.path.insert(0, "tests")
@@ -9,28 +9,14 @@ L = _lib.lib()
 st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 i64 = ctypes.c_int64
 torch.manual_seed(0)
-for (M, N, K, f16, bias) in [(256, 256, 64, 0, False), (1000, 512, 192, 1, True), (4096, 3072, 768, 0, True), (70, 256, 128, 1, False),
-                             (102400, 3072, 768, 0, False)]:
-    dt = torch.float16 if f16 else torch.bfloat16
-    A = torch.randn(M, K, device="cuda").to(dt)
-    B = (torch.randn(N, K, device="cuda") * 0.05).to(dt)
-    bs = torch.randn(N, device="cuda") if bias else None
-    C = torch.full((M, N), float("nan"), device="cuda")
-    r = L.svb_gemm_persistent(ptr(A), ptr(B), ptr(C), ptr(bs), M, N, K, i64(K), i64(K), i64(N), f16, st)
-    torch.cuda.synchronize()
-    assert r == 0, L.svb_last_error()
-    rows = torch.arange(0, M, max(1, M // 512), device="cuda")
-    ref = A[rows].float() @ B.float().t() + (bs if bias else 0)
-    err = (C[rows] - ref).abs().max().item() / ref.abs().max().item()
-    print(f"M={M} N={N} K={K} f16={f16} bias={bias}: rel err {err:.2e}  nan {torch.isnan(C).any().item()}")
-    assert err < 2e-5 and not torch.isnan(C).any()
 M, N, K = 102400, 3072, 768
 A = torch.randn(M, K, device="cuda").to(torch.bfloat16)
 B = (torch.randn(N, K, device="cuda") * 0.05).to(torch.bfloat16)
 C = torch.empty(M, N, device="cuda")
 PA = (ctypes.c_void_p * 1)(A.data_ptr()); PB = (ctypes.c_void_p * 1)(B.data_ptr())
 def t(fn, n=10):
-    for _ in range(3): fn()
+    assert fn() == 0, L.svb_last_error()
+    for _ in range(2): fn()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()

@@ -785,30 +785,6 @@ def test_overlapped_reducer_orders_reductions_before_autograd(svb, net):
     net.zero_grad()
 
 
-@pytest.mark.parametrize("M,N,K,f16,bias", [(256, 256, 64, 0, False), (1000, 512, 192, 1, True), (70, 256, 128, 1, False),
-                                            (5000, 3072, 768, 0, True)])
-def test_persistent_input_gemm(svb, M, N, K, f16, bias):
-    """svb_gemm_persistent (csrc/pgemm.cu: the LSTM input projection W_ih x_t as one batched GEMM) against fp32 matmul
-    on the same bf16 / fp16-rounded operands: ragged M (rows clipped by TMA), bias, several tiles per CTA pair."""
-    import ctypes
-    from pytorch_speaker_verification_b200 import _lib
-    from pytorch_speaker_verification_b200._lib import ptr
-    g = torch.Generator(device="cuda").manual_seed(M + N + K)
-    dt = torch.float16 if f16 else torch.bfloat16
-    A = torch.randn(M, K, device="cuda", generator=g).to(dt)
-    B = (torch.randn(N, K, device="cuda", generator=g) * 0.05).to(dt)
-    bs = torch.randn(N, device="cuda", generator=g) if bias else None
-    C = torch.full((M, N), float("nan"), device="cuda")
-    i64 = ctypes.c_int64
-    r = _lib.lib().svb_gemm_persistent(ptr(A), ptr(B), ptr(C), ptr(bs), M, N, K, i64(K), i64(K), i64(N), f16,
-                                       ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
-    assert r == 0
-    ref = A.float() @ B.float().t() + (bs if bias else 0.0)
-    assert not torch.isnan(C).any()
-    assert float((C - ref).abs().max() / ref.abs().max()) < 2e-5
-    assert _lib.lib().svb_gemm_persistent(ptr(A), ptr(B), ptr(C), None, M, 100, K, i64(K), i64(K), i64(N), f16, None) != 0
-
-
 # ----------------------------------------------------------------------------------------------- optimizer tail
 def test_fused_clip_sgd_matches_clip_grad_norm_and_sgd(svb, net):
     """svb.FusedClipSGD (csrc/optim.cu) against the torch entry points train_speech_embedder.py:63-65 calls
