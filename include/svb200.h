@@ -350,6 +350,45 @@ int svb_segment_mean(const float* emb, int D, const int* seg_offsets, int P, dou
 int svb_logmel(const float* y, int64_t n, int hop, const float* window, int w0, int w1, const float* twiddle,
                const float* mel_w, int nmels, float* out, int n_frames, void* stream);
 
+/* ---- TI-SV training-set preprocessing (data_preprocess.py save_spectrogram_tisv; new: DESIGN.md 4.8) ---------------
+ * Silence split, librosa 0.6 effects.split(y, top_db, ref=np.max, frame_length=2048, hop_length=512), for a signal y of
+ * n > 1024 samples:
+ *   pad y with 1024 samples on each side, reflecting without repeating the edge sample (np.pad(mode="reflect"));
+ *   F = 1 + n / 512 frames; frame t covers padded samples [512 t, 512 t + 2048) and p_t = the mean of their squares,
+ *   in float64 (the squares of float32 samples are exact) with a fixed order: per 512-sample block a fixed sum, then
+ *   p_t = ((B_t + B_t+1) + (B_t+2 + B_t+3)) / 2048;
+ *   frame t is non-silent iff 10 log10(max(1e-10, p_t)) - 10 log10(max(1e-10, max_t p_t)) > -top_db;
+ *   the interval edges are the frames t where the mask changes (frames outside [0, F) count as silent), times 512,
+ *   clipped to n, paired as half-open [start, end).
+ * So an all-zero signal is one interval [0, n), top_db <= 0 gives none, and a last interval may be empty ([n, n] when
+ * n % 512 == 0).  librosa >= 0.10 pads with zeros instead, which can change frames 0 and F - 1 only.
+ * Signals with n <= 1024 give no interval.  Interval counts of one signal are at most (F + 1) / 2. */
+
+/* Bytes of svb_split_nonsilent's workspace: (4 n_signals + total_samples / 512) doubles of block sums. */
+int svb_split_workspace_bytes(int64_t total_samples, int n_signals, size_t* bytes);
+/* The intervals of n_signals signals concatenated in y: signal i is y[offsets[i], offsets[i+1]) (offsets: device,
+ * n_signals + 1 ascending int64, offsets[0] = 0, offsets[n_signals] = total_samples).  Only intervals with
+ * end - start >= min_len are kept (min_len = 0 keeps every one; data_preprocess.py's `> utter_min_len` is
+ * min_len = floor(utter_min_len) + 1).  Signal i's kept intervals go, in order, to the int64 pairs
+ * intervals[2 slot_offsets[i] ...] (sample offsets within the signal); slot_offsets (device, n_signals int64) must
+ * leave (F_i + 1) / 2 pairs to signal i (F_i = 0 for n_i <= 1024).  counts[i] (device int64) = the number of kept
+ * intervals, or -1 when signal i holds a non-finite sample.  Two launches; no allocation, synchronisation or float
+ * atomics: identical from run to run and across streams.  SVB_ERR_ARG before any launch unless n_signals >= 0,
+ * total_samples >= 0, min_len >= 0, top_db is not NaN, the pointers are non-null and the workspace is 8-byte aligned
+ * and large enough. */
+int svb_split_nonsilent(const float* y, const int64_t* offsets, int n_signals, int64_t total_samples, double top_db,
+                        int64_t min_len, const int64_t* slot_offsets, void* workspace, size_t workspace_bytes,
+                        int64_t* intervals, int64_t* counts, void* stream);
+/* Log-mel frames of many segments of y in one launch, the same device code and bits as svb_logmel on the segment:
+ * rows (device, P x 3 int64) = {segment start in y, segment length L >= 1, first frame f0}; out (P, nmels,
+ * frames_per_row) float32, out[p, :, j] = frame f0 + j of svb_logmel(y + start, L, ...), the reflect padding taken at
+ * the segment's bounds (repeatedly when a frame reaches more than L - 1 samples past them, as np.pad does).  The
+ * caller keeps f0 + frames_per_row <= 1 + L / hop when it wants frames librosa would give.  Other arguments as
+ * svb_logmel.  SVB_ERR_ARG before any launch unless P >= 0, frames_per_row >= 1, hop >= 1, nmels >= 1,
+ * 0 <= w0 < w1 <= 512, the pointers are non-null (P > 0) and P * frames_per_row < 2^34. */
+int svb_logmel_frames(const float* y, const int64_t* rows, int64_t P, int frames_per_row, int hop, const float* window,
+                      int w0, int w1, const float* twiddle, const float* mel_w, int nmels, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -14,4 +14,4 @@ from .calibration import (Calibration, CalibrationMetrics,             # noqa: F
 from .dvector import align_embeddings, extract_dvectors, get_windows  # noqa: F401
 from .optim import FusedClipSGD                                       # noqa: F401
 from .staging import prefetch                                         # noqa: F401
-from .frontend import log_mel_spectrogram                              # noqa: F401
+from .frontend import log_mel_spectrogram, split_nonsilent, tisv_spectrograms  # noqa: F401

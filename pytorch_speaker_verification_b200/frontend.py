@@ -5,6 +5,11 @@ Host mirror of data_preprocess.py:41-45 / dvector_create.py:43-47 (librosa.core.
 The tables (periodic Hann window padded to n_fft, DFT twiddles, Slaney mel filterbank) are built once per device in
 float64 and handed to svb_logmel; the arithmetic runs in libsvb200.so (csrc/frontend.cu), no CPU fallback.
 Parity is unpinned: librosa is not available where this was built, see oracle/frontend.py.
+
+The TI-SV training set of data_preprocess.py (save_spectrogram_tisv: librosa.effects.split, the utter_min_len filter,
+first and last tisv_frame frames of each kept interval) is built by tisv_spectrograms for many utterances at once:
+one split launch pair over all signals (csrc/preprocess.cu), one host read of the kept intervals, one log-mel launch
+over every output frame (svb_logmel_frames, the same device code as svb_logmel).  DESIGN.md 4.8.
 """
 import math
 
@@ -12,6 +17,7 @@ import numpy as np
 import torch
 
 from . import ops
+from .dvector import _pool
 
 N_FFT = 512
 _tables = {}
@@ -66,3 +72,123 @@ def log_mel_spectrogram(y, sr=16000, win_length=400, hop=160, n_mels=40):
         win, w0, w1, tw, melw = _get_tables(dev, sr, win_length, n_mels)
         out = torch.ops.svb200.logmel(yg, win, tw, melw, int(hop), w0, w1)
     return out
+
+
+# ------------------------------------------------------------------------------------------ TI-SV preprocessing
+SPLIT_HOP = 512           # librosa.effects.split defaults: frame_length 2048, hop_length 512
+
+
+def _signal(s, i):
+    t = s if isinstance(s, torch.Tensor) else torch.as_tensor(np.asarray(s))
+    if t.dim() != 1:
+        raise ValueError(f"signal {i} must be 1-D, got shape {tuple(t.shape)}")
+    if not t.is_floating_point():
+        raise ValueError(f"signal {i} must hold floating-point samples, got {t.dtype}")
+    return t.detach()
+
+
+def _split(signals, top_db, min_len):
+    """Stage the signals into one float32 device buffer and run svb_split_nonsilent once.
+    -> (device samples, offsets, kept intervals (K, 2) int64 of all signals in order, counts per signal)."""
+    ts = [_signal(s, i) for i, s in enumerate(signals)]
+    dev = ops._target_device(*ts)
+    ns = len(ts)
+    n = np.asarray([t.numel() for t in ts], dtype=np.int64)
+    offsets = np.concatenate([[0], np.cumsum(n)]).astype(np.int64)
+    frames = np.where(n > 2 * SPLIT_HOP, 1 + n // SPLIT_HOP, 0)
+    slots = (frames + 1) // 2
+    slot_offsets = np.concatenate([[0], np.cumsum(slots)[:-1]]).astype(np.int64)
+    n_slots = int(slots.sum())
+    host = [not t.is_cuda for t in ts]
+    total_host = int(sum(int(k) for k, h in zip(n, host) if h))
+    # one page-locked buffer, one copy: [offsets | slot offsets | samples of the signals that live on the host]
+    nb_tab = 8 * (2 * ns + 1)
+    buf = _pool.take(nb_tab + 4 * total_host)
+    try:
+        tab = buf[:nb_tab].view(torch.int64)
+        tab[:ns + 1] = torch.from_numpy(offsets)
+        tab[ns + 1:] = torch.from_numpy(slot_offsets)
+        hs = buf[nb_tab:nb_tab + 4 * total_host].view(torch.float32)
+        o = 0
+        for t, h in zip(ts, host):
+            if h:
+                hs[o:o + t.numel()].copy_(t)
+                o += t.numel()
+        with torch.cuda.device(dev):
+            g = buf[:nb_tab + 4 * total_host].to(dev, non_blocking=True)
+            gtab = g[:nb_tab].view(torch.int64)
+            gs = g[nb_tab:].view(torch.float32)
+            if all(host):
+                y = gs
+            else:
+                parts, o = [], 0
+                for t, h in zip(ts, host):
+                    if h:
+                        parts.append(gs[o:o + t.numel()])
+                        o += t.numel()
+                    else:
+                        parts.append(t.to(torch.float32).reshape(-1))
+                y = torch.cat(parts)
+            res = torch.ops.svb200.split_nonsilent(y, gtab[:ns + 1], gtab[ns + 1:], n_slots, top_db, min_len).cpu().numpy()
+    finally:
+        torch.cuda.current_stream(dev).synchronize()               # the copy out of `buf` has finished
+        _pool.give(buf)
+    counts = res[2 * n_slots:]
+    bad = np.flatnonzero(counts < 0)
+    if bad.size:
+        raise ValueError(f"signal {int(bad[0])} holds a non-finite sample")
+    K = int(counts.sum())
+    first = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64)
+    pairs = res[:2 * n_slots].reshape(n_slots, 2)
+    idx = np.repeat(slot_offsets, counts) + np.arange(K, dtype=np.int64) - np.repeat(first, counts)
+    return y, offsets, pairs[idx], counts
+
+
+def split_nonsilent(y, top_db=60):
+    """librosa.effects.split(y, top_db) (librosa 0.6: ref=np.max, frame_length 2048, hop_length 512) of one 1-D signal on
+    any device -> (K, 2) int64 numpy array of the non-silent intervals [start, end).  Definitions in
+    include/svb200.h; librosa >= 0.10 pads with zeros instead of reflecting, which can change the first and last
+    frames only.  Raises ValueError for a signal of 1024 samples or fewer, or a non-finite sample."""
+    t = _signal(y, 0)
+    if t.numel() <= 2 * SPLIT_HOP:
+        raise ValueError(f"the silence split needs more than 1024 samples, got {t.numel()}")
+    return _split([t], float(top_db), 0)[2]
+
+
+@torch.no_grad()
+def tisv_spectrograms(signals, sr=16000, window=0.025, hop=0.01, nmels=40, tisv_frame=180, top_db=30):
+    """The TI-SV training features of data_preprocess.py's save_spectrogram_tisv for many utterances at once.
+
+    For each signal, in order: the non-silent intervals of split_nonsilent(y, top_db); those longer than
+    utter_min_len = (tisv_frame * hop + window) * sr samples; for each, the log-mel spectrogram of the interval alone
+    (reflect padding at the interval's bounds, n_fft 512, win_length int(window * sr), hop_length int(hop * sr)), its
+    first tisv_frame frames, then its last tisv_frame frames (they overlap when the interval has fewer than
+    2 * tisv_frame frames).  ``signals``: a list of 1-D arrays or tensors on any device, any float dtype.
+    Returns (spec, counts): spec (P, nmels, tisv_frame) float32 CUDA tensor, which for one speaker's utterances is the
+    reference's np.array(utterances_spec) (shape (0, nmels, tisv_frame) where it has none); counts[i] the rows signal i
+    contributed (int64 numpy).  Signals of 1024 samples or fewer contribute nothing.  One host read; ValueError for a
+    non-1-D signal, a non-finite sample, or a config that does not give 1 <= hop <= window <= 512 samples."""
+    win_length, hop_length = int(window * sr), int(hop * sr)
+    if not 1 <= hop_length <= win_length <= N_FFT:
+        raise ValueError(f"window {window} s and hop {hop} s at {sr} Hz give win_length {win_length} and hop_length "
+                         f"{hop_length} samples: need 1 <= hop_length <= win_length <= {N_FFT}")
+    if int(tisv_frame) != tisv_frame or tisv_frame < 1 or int(nmels) != nmels or nmels < 1:
+        raise ValueError(f"tisv_frame and nmels must be positive integers, got {tisv_frame} and {nmels}")
+    T, nmels = int(tisv_frame), int(nmels)
+    utter_min_len = (tisv_frame * hop + window) * sr          # data_preprocess.py's expression, kept iff L > it
+    min_len = math.floor(utter_min_len) + 1
+    if len(signals) == 0:
+        return torch.empty(0, nmels, T, device=ops._dev()), np.zeros(0, dtype=np.int64)
+    y, offsets, iv, counts = _split(signals, float(top_db), min_len)
+    dev = y.device
+    sig = np.repeat(np.arange(len(counts)), counts)
+    start, length = offsets[sig] + iv[:, 0], iv[:, 1] - iv[:, 0]
+    rows = np.empty((2 * len(iv), 3), dtype=np.int64)
+    rows[0::2, 0] = rows[1::2, 0] = start
+    rows[0::2, 1] = rows[1::2, 1] = length
+    rows[0::2, 2] = 0
+    rows[1::2, 2] = 1 + length // hop_length - T
+    with torch.cuda.device(dev):
+        win, w0, w1, tw, melw = _get_tables(dev, sr, win_length, nmels)
+        spec = torch.ops.svb200.logmel_frames(y, torch.from_numpy(rows).to(dev), win, tw, melw, T, hop_length, w0, w1)
+    return spec, 2 * counts

@@ -1025,7 +1025,56 @@ def _logmel(y: torch.Tensor, window: torch.Tensor, twiddle: torch.Tensor, mel_w:
 _op("logmel(Tensor y, Tensor window, Tensor twiddle, Tensor mel_w, int hop, int w0, int w1) -> Tensor", _logmel,
     lambda y, window, twiddle, mel_w, hop, w0, w1: y.new_empty(mel_w.shape[0], 1 + y.numel() // hop))
 
+
+# ------------------------------------------------------------------------------------------ TI-SV preprocessing
+# split_nonsilent out (2 * n_slots + n_signals int64): the interval pairs of every signal's slot range, then the
+# per-signal counts (-1: a non-finite sample), so that one host read fetches both (include/svb200.h)
+def _split_nonsilent(y: torch.Tensor, offsets: torch.Tensor, slot_offsets: torch.Tensor, n_slots: int, top_db: float,
+                     min_len: int) -> torch.Tensor:
+    if y.dtype != torch.float32 or y.dim() != 1 or offsets.dtype != torch.int64 or slot_offsets.dtype != torch.int64:
+        raise ValueError("split_nonsilent expects float32 samples (total,) and int64 offsets")
+    if offsets.dim() != 1 or offsets.numel() < 1 or slot_offsets.shape != (offsets.numel() - 1,):
+        raise ValueError("split_nonsilent expects offsets (n_signals + 1,) and slot_offsets (n_signals,)")
+    _same_device("split_nonsilent", y, offsets, slot_offsets)
+    ns, total = int(offsets.numel()) - 1, int(y.numel())
+    out = torch.empty(2 * int(n_slots) + ns, dtype=torch.int64, device=y.device)
+    if ns == 0:
+        return out
+    with torch.cuda.device(y.device):
+        nbytes = _sz(0)
+        check(_lib.lib().svb_split_workspace_bytes(_i64(total), ns, ctypes.byref(nbytes)), "svb_split_workspace_bytes")
+        ws = torch.empty(nbytes.value, dtype=torch.uint8, device=y.device)
+        yc = y.contiguous() if total else y.new_zeros(1)
+        check(_lib.lib().svb_split_nonsilent(ptr(yc), ptr(offsets.contiguous()), ns, _i64(total),
+                                             ctypes.c_double(top_db), _i64(min_len), ptr(slot_offsets.contiguous()),
+                                             ptr(ws), _sz(nbytes.value), ptr(out), ptr(out[2 * int(n_slots):]),
+                                             stream_ptr(y.device)), "svb_split_nonsilent")
+    return out
+
+
+def _logmel_frames(y: torch.Tensor, rows: torch.Tensor, window: torch.Tensor, twiddle: torch.Tensor,
+                   mel_w: torch.Tensor, frames: int, hop: int, w0: int, w1: int) -> torch.Tensor:
+    if y.dtype != torch.float32 or rows.dtype != torch.int64 or rows.dim() != 2 or rows.shape[1] != 3:
+        raise ValueError("logmel_frames expects float32 samples and int64 rows (P, 3)")
+    _same_device("logmel_frames", y, rows, window, twiddle, mel_w)
+    P, nmels = int(rows.shape[0]), int(mel_w.shape[0])
+    out = torch.empty(P, nmels, int(frames), dtype=torch.float32, device=y.device)
+    with torch.cuda.device(y.device):
+        check(_lib.lib().svb_logmel_frames(ptr(y.contiguous()), ptr(rows.contiguous()), _i64(P), int(frames), int(hop),
+                                           ptr(window), int(w0), int(w1), ptr(twiddle), ptr(mel_w), nmels, ptr(out),
+                                           stream_ptr(y.device)), "svb_logmel_frames")
+    return out
+
+
+_op("split_nonsilent(Tensor y, Tensor offsets, Tensor slot_offsets, int n_slots, float top_db, int min_len) -> Tensor",
+    _split_nonsilent, lambda y, offsets, slot_offsets, n_slots, top_db, min_len:
+    y.new_empty(2 * n_slots + offsets.shape[0] - 1, dtype=torch.int64))
+_op("logmel_frames(Tensor y, Tensor rows, Tensor window, Tensor twiddle, Tensor mel_w, int frames, int hop, int w0, "
+    "int w1) -> Tensor", _logmel_frames,
+    lambda y, rows, window, twiddle, mel_w, frames, hop, w0, w1: y.new_empty(rows.shape[0], mel_w.shape[0], frames))
+
 OP_NAMES = ["pack_weights", "embedder_fwd", "embedder_bwd", "ge2e_loss", "ge2e_rows", "scale3", "centroids", "centroids_bwd",
             "utterance_centroids", "cossim", "cossim_bwd", "calc_loss", "calc_loss_bwd", "eer_counts", "eer_sweep", "peer_gather", "peer_reduce",
             "eer_finish", "verif_metrics", "verif_metrics_sim", "cohort_stats", "cohort_stats_scores", "score_trials",
-            "asnorm_sim", "calib_metrics", "calib_train", "dvector_windows", "segment_mean", "clip_sgd", "logmel"]
+            "asnorm_sim", "calib_metrics", "calib_train", "dvector_windows", "segment_mean", "clip_sgd", "logmel",
+            "split_nonsilent", "logmel_frames"]
