@@ -96,9 +96,10 @@ int svb_set_persistent(int on);
  * one cooperative cluster launch, split-K over 4-CTA clusters with a DSMEM reduction) when H == 768 and L <= 3;
  * 0 = one fused GEMM + gate-backward launch per frame and batched dX GEMMs. */
 int svb_set_persistent_bwd(int on);
-/* Large-batch GE2E / get_cossim (rows x centroids >= 2^18, D % 64 == 0): 1 (default) = the three contractions run on
- * tensor cores as 3-term split-fp16 products between the phase kernels, 0 = fp32 SIMT contractions (one cooperative
- * launch).  Both agree with the float64 oracle to 1e-5 (utils.py:72-115,126-132). */
+/* Large-batch GE2E / get_cossim (rows x centroids >= 2^18, D % 64 == 0, D <= 256): 1 (default) = the three
+ * contractions run on tensor cores as 3-term split-fp16 products between the phase kernels, 0 = fp32 SIMT contractions
+ * (one cooperative launch).  Both agree with the float64 oracle to 1e-5 (utils.py:72-115,126-132).  Wider D always
+ * takes the SIMT contractions: the tensor-core accumulation's bias grows with D (ge2e.cu, kTcMaxD). */
 int svb_set_ge2e_tensor_cores(int on);
 
 /* ---- multi-GPU GE2E exchange over NVLink peer memory (new: the reference, speech_embedder_net.py:43-49, is

@@ -81,7 +81,8 @@ def _f32(t, *shape):
 
 # ------------------------------------------------------------------------------------------ debug switches
 def set_poison_workspace(on):
-    """Debug: NaN-fill every forward workspace, so that a kernel reading a slot before it is written shows up."""
+    """Debug: NaN-fill every forward workspace (and the GE2E outputs), so that a kernel reading a slot before it is
+    written, or leaving an output element unwritten, shows up."""
     global _POISON
     _POISON = bool(on)
 
@@ -365,6 +366,10 @@ def _ge2e_call(E, Cext, w, b, dcos, gscale, want_cos, want_loss, need_grad, fuse
         dw = torch.empty((), **f32) if (need_grad and w is not None) else None
         db = torch.empty((), **f32) if (need_grad and w is not None) else None
         lsum = torch.empty((), **f32) if want_loss else None
+        if _POISON:          # debug: NaN-fill the workspace and every output, so that a slot no kernel writes shows
+            for t in (ws, cos, per, dE, dC, dw, db, lsum):
+                if t is not None:
+                    t.view(-1).view(torch.uint8).fill_(255)
         check(_lib.lib().svb_ge2e_ex(ptr(E), ptr(Cext), N, M, D, Nc, ptr(w), ptr(b), ptr(dcos), ptr(gscale), ptr(cos),
                                      ptr(per), ptr(lsum), ptr(dE), ptr(dC), ptr(dw), ptr(db), ptr(ws), _sz(nbytes.value),
                                      int(fused), int(loss), stream_ptr(dev)), "svb_ge2e_ex")
@@ -407,6 +412,9 @@ def _ge2e_rows(E: torch.Tensor, C: torch.Tensor, w: torch.Tensor, b: torch.Tenso
         # one buffer for everything that is summed over the ranks: dC (Nc, D), then loss, dw, db
         red = torch.empty(Nc * D + 3, dtype=torch.float32, device=dev)
         dE = torch.empty(N, M, D, dtype=torch.float32, device=dev)
+        if _POISON:          # debug: NaN-fill the workspace and the outputs (see _ge2e_call)
+            for t in (ws, red, dE):
+                t.view(-1).view(torch.uint8).fill_(255)
         base = red.data_ptr()
         f = lambda off: ctypes.c_void_p(base + 4 * off)
         check(_lib.lib().svb_ge2e_rows_ex(ptr(E.contiguous()), ptr(C.contiguous()), N, M, D, Nc, int(col0),

@@ -9,7 +9,6 @@ so that a slot read before it is written shows up.
 Bars are the suite's (test_gpu_parity.py): embeddings 1e-3 worst per-row L2-relative; parameter gradients 1.2e-2
 (weights) and 3e-2 (biases) per-tensor L2-relative, for the loss (e * v).sum() with a fixed random v.
 """
-import ctypes
 import os
 from contextlib import contextmanager
 
@@ -19,6 +18,7 @@ import torch
 
 import _inputs as I
 from _embedder_shapes import BY_ID, CASES, narrow_kz6, param_names, wgrad_overlap
+from _launches import count_launches, launched
 from oracle import embedder as oemb
 
 pytestmark = pytest.mark.gpu
@@ -166,31 +166,6 @@ def test_embedder_matches_float64_oracle(svb, models, oracle, case, B, T):
         print(f"\n[{case.id} I={case.nmels} H={case.hidden} L={case.num_layer} P={case.proj} B={B} T={T} "
               f"{'persistent' if persistent else 'per-frame'}] emb {err:.2e}  worst weight grad {ew:.2e}  "
               f"worst bias grad {eb:.2e}")
-
-
-def count_launches(fn):
-    """-> {kernel (mangled name): launches} of this library during fn(), or None when CUPTI cannot be used."""
-    from pytorch_speaker_verification_b200 import _lib
-    L = _lib.lib()
-    if L.svb_launch_count_begin() != 0:
-        return None
-    try:
-        fn()
-        torch.cuda.synchronize()
-    finally:
-        ours, other = ctypes.c_longlong(0), ctypes.c_longlong(0)
-        names = ctypes.create_string_buffer(1 << 16)
-        L.svb_launch_count_end(ctypes.byref(ours), ctypes.byref(other), names, ctypes.c_size_t(len(names)))
-    per = {}
-    for item in names.value.decode().split(";"):
-        if "=" in item:
-            k, n = item.rsplit("=", 1)
-            per[k] = int(n)
-    return per
-
-
-def launched(names, *parts):
-    return any(all(p in k for p in parts) for k in names)
 
 
 def assert_routes(case, B, T, names):

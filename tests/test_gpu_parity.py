@@ -676,7 +676,8 @@ def test_centroid_kernels_bit_exact(svb):
         svb.utils.get_utterance_centroids(torch.randn(3, 1, 8))
 
 
-@pytest.mark.parametrize("N,M,D,shards", [(8, 4, 32, 2), (64, 10, 256, 8), (512, 10, 256, 8), (12, 3, 20, 3)])
+@pytest.mark.parametrize("N,M,D,shards", [(8, 4, 32, 2), (64, 10, 256, 8), (512, 10, 256, 8), (12, 3, 20, 3),
+                                          (264, 16, 192, 2)])
 def test_ge2e_row_shards_sum_to_the_global_batch(svb, N, M, D, shards):
     """svb_ge2e_rows (multi-GPU design A: a rank's rows against the all-gathered centroids) on one GPU: the shards'
     partial losses / dw / db / centroid gradients sum to the global batch's (fp64 closed form), and
@@ -689,10 +690,15 @@ def test_ge2e_row_shards_sum_to_the_global_batch(svb, N, M, D, shards):
     C = svb.get_centroids(E)
     nl = N // shards
     reds, dEs = [], []
-    for r in range(shards):
-        red, dE = torch.ops.svb200.ge2e_rows(E[r * nl:(r + 1) * nl].contiguous(), C, w, b, r * nl)
-        reds.append(red.double())
-        dEs.append(dE)
+    from pytorch_speaker_verification_b200 import ops
+    try:
+        ops.set_poison_workspace(True)              # workspace and outputs start as NaN: every element must be written
+        for r in range(shards):
+            red, dE = torch.ops.svb200.ge2e_rows(E[r * nl:(r + 1) * nl].contiguous(), C, w, b, r * nl)
+            reds.append(red.double())
+            dEs.append(dE)
+    finally:
+        ops.set_poison_workspace(False)
     red = torch.stack(reds).sum(dim=0)
     dC = red[:N * D].view(N, D).float()
     assert rel(red[N * D].item(), o["loss"]) < 1e-5
